@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm
     python bench.py --impl reference --gpus N --steps K --warmup W   # CPU reference arm
+    python bench.py --gpus N --steps K --warmup W --dump-outputs DIR  # + the last timed step's logits in DIR
 
 A "step" is one pass of the hot path (frames on device -> logits on device) over
 one batch of synthetic event frames.  Workload at N GPUs = BASELINE.json
@@ -36,6 +37,7 @@ GOP_PER_SAMPLE_T20 = 33.647      # dense-equivalent int8 GOP / sample (BASELINE.
 CONV2_GOP_PER_SAMPLE = 2 * 12.080
 METRIC = "TCJA-SNN inference samples/sec (T=20)"
 UNIT = "samples/s"
+DUMP_MAX_BYTES = 48 << 20          # --dump-outputs: larger outputs are sampled (keeps a dump easy to store and compare)
 
 
 def peaks():
@@ -280,6 +282,8 @@ def run_ours(args):
   D.reduce_max(t)
   ms_max = float(t.item())
   value = B * ws * args.steps / (ms_max / 1e3)
+  if args.dump_outputs:
+    dump_logits(args.dump_outputs, D.gather_logits(logits, B * ws), rank)
 
   # ---- end to end: pinned host frames -> H2D -> forward -> logits D2H ------
   # the public host-memory call: chunked H2D on a copy stream overlapped with compute, logits copied back
@@ -383,6 +387,21 @@ def run_ours(args):
   if torch.distributed.is_initialized():
     torch.distributed.destroy_process_group()
   return 0
+
+
+def dump_logits(out_dir, logits, rank):
+  """What the timed path hands its caller in the last timed step: the logits of the global batch in sample order, as
+  DIR/logits.npy (float32).  The inputs are seeded, so two builds run with the same arguments can be compared output
+  for output.  Beyond DUMP_MAX_BYTES a fixed, seeded sample of rows (in sample order) is written."""
+  import numpy as np
+  if rank != 0:
+    return
+  x = logits.cpu().numpy()
+  if x.nbytes > DUMP_MAX_BYTES:
+    rows = np.random.default_rng(0).choice(x.shape[0], DUMP_MAX_BYTES // x[0].nbytes, replace=False)
+    x = x[np.sort(rows)]
+  os.makedirs(out_dir, exist_ok=True)
+  np.save(os.path.join(out_dir, "logits.npy"), x)
 
 
 def dominant_kernel_roofline(eng, frames, args, dev):
@@ -516,7 +535,13 @@ def main():
   ap.add_argument("--cpu-batch", type=int, default=16)
   ap.add_argument("--ref-batch", type=int, default=16)
   ap.add_argument("--no-cpu-baseline", action="store_true")
+  ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                  help="after the timed steps, write the logits of the last one to DIR/logits.npy (float32)")
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error("--steps must be at least 1")
+  if args.dump_outputs and args.impl == "reference":
+    ap.error("--dump-outputs applies to --impl ours (the reference arm's sample size follows its timing)")
   if args.warmup < 3 and args.impl == "ours":
     args.warmup = 3
   if args.impl == "reference":

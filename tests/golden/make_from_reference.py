@@ -246,7 +246,7 @@ def network_fixture(quant, sl, models, bits, p, T, H, B, seed_w, seed_x, num_cla
   import flax.linen as nn
   import jax.nn
   import ml_collections
-  sys.path.insert(0, ROOT)
+  sys.path[:0] = [ROOT, os.path.dirname(HERE)]
   from snnquantprune_b200 import synthetic
   v = synthetic.make_variables(bits=bits, prune_percentage=p, T=T, H=H, seed=seed_w, num_classes=num_classes, stable=True)
   frames = synthetic.make_frames(B, T, H, H, seed=seed_x, stable=True)
@@ -301,6 +301,13 @@ def network_fixture(quant, sl, models, bits, p, T, H, B, seed_w, seed_x, num_cla
       keep = s8 if n in ("conv4", "conv5") else pooled                  # what the next layer / TCJA consumes
       fx[f"{n}_bits"] = np.packbits(keep.reshape(-1))      # complete: per-layer teacher forcing needs every input spike
       fx[f"{n}_bits_shape"] = np.array(keep.shape)
+      if full and n == "conv1":
+        # stored as the difference to the oracle's conv1 and the digest (tests/reffix.py load_network rebuilds it):
+        # the bits themselves would take the file over 1 MB
+        import reffix
+        diff = np.flatnonzero(reffix.oracle_conv1_pooled(v, bits, frames).reshape(-1) != keep.reshape(-1))
+        fx[f"{n}_bits_sha"] = np.array(sha(fx.pop(f"{n}_bits")))
+        fx[f"{n}_bits_diff"] = diff.astype(np.int64)
       st = max(1, uT.shape[1] // 8)                                  # 8 x 8 sub-grid of final membranes
       fx[f"{n}_uT"] = np.ascontiguousarray(uT[:, ::st, ::st, :], F32)
       fx[f"{n}_uT_stride"] = np.array(st)
