@@ -163,7 +163,14 @@ typedef struct snnqp_block_params {
  *          folded into two fp16 weight pieces, bias on a constant-one K
  *          column) and the epilogue only compares, resets and packs.  The
  *          accumulation rounding is the tensor core's, not IEEE fma: tolerance
- *          parity (membrane 1e-5, spike flips <= 1e-4), not bit parity. */
+ *          parity (membrane 1e-5, spike flips <= 1e-4), not bit parity.
+ *          Envelope: all 128 channels share one power-of-two domain scale,
+ *          fitted to the largest 63.5 * |scale| or |bias| / 2 (fully pruned
+ *          channels included).  A channel ~100x the others (all weights
+ *          pruned, running var 0) stays inside both bars; with one channel
+ *          2^16 or 2^20 times the others the flip bar still holds but some
+ *          membranes miss 1e-5 (up to 2.3e-4 relative, no flipped spike,
+ *          measured on a B200).  Use EXACT or FAST for such checkpoints. */
 #define SNNQP_LIF_TENSOR 2
 
 /* SpikingBlock(QuantConv 3x3 pad 1, BatchNorm, multi_step_LIF) over T steps

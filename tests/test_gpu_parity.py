@@ -125,9 +125,10 @@ def test_fold_affine_bit_exact(cuda_lib):
 
 # ------------------------------------------------------- fused conv block ----
 def run_conv(lib, x_tb, wq, scale, bias, Cout, pool, impl, att=None, tau=2.0, batch_major=False, counts=None,
-             dumps=True, x_bits=False, y_bits=False, lif_mode=0):
+             dumps=True, x_bits=False, y_bits=False, lif_mode=0, popcount=None):
   """x_tb: numpy (T,B,H,W,Cin) u8.  Calls snnqp_spiking_conv3x3_fwd through the
-  C-ABI; returns numpy (spikes (T,B,Ho,Wo,C), u (B,H,W,C), acc (T,B,H,W,C))."""
+  C-ABI; returns numpy (spikes (T,B,Ho,Wo,C), u (B,H,W,C), acc (T,B,H,W,C)).
+  ``popcount``: optional int32 CUDA tensor [B][T] passed as y_popcount."""
   T, B, H, W, Cin = x_tb.shape
   if x_bits:
     x_tb = np.packbits(x_tb, axis=-1, bitorder="little")          # SNNQP_SPIKES_BITS
@@ -153,6 +154,8 @@ def run_conv(lib, x_tb, wq, scale, bias, Cout, pool, impl, att=None, tau=2.0, ba
   p.tau, p.v_threshold, p.v_reset = tau, 1.0, 0.0
   p.pool, p.impl = int(pool), impl
   p.x_format, p.y_format, p.lif_mode = int(x_bits), int(y_bits), lif_mode
+  if popcount is not None:
+    p.y_popcount = P(popcount)
   ud, accd = (u, acc) if dumps else (None, None)      # no instrumentation outputs -> the production (FAST) variant
   if dumps == "u":                                     # membranes only (conv1's LIF_TENSOR kernel has no accumulator dump)
     accd = None
