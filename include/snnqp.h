@@ -154,7 +154,12 @@ typedef struct snnqp_block_params {
  *          bit-identical to the oracle;
  *   FAST   fma(u, 0.5, x / 2) with the halving folded into scale / bias: one
  *          rounding instead of two, |du| <= 1 ulp per step (north-star bar
- *          1e-5), spikes may flip only when un is within an ulp of 1. */
+ *          1e-5), spikes may flip only when un is within an ulp of 1.
+ *          Tested against a float64 band: per step h = fma(acc, s/2, b/2)
+ *          and un = fma(u, 0.5, h) round once each, e_t = 2^-24 (|h| + |un|),
+ *          delta_t = e_t + delta_{t-1} / 2 until the first step with
+ *          |un - 1| <= delta_t; every pooled spike the band decides must
+ *          equal float64 (tests/test_gpu_conv1_rounding_band.py). */
 #define SNNQP_LIF_EXACT 0
 #define SNNQP_LIF_FAST 1
 /*   TENSOR (conv1, tcgen05 path, production variant only; EXACT elsewhere): the
@@ -164,13 +169,26 @@ typedef struct snnqp_block_params {
  *          column) and the epilogue only compares, resets and packs.  The
  *          accumulation rounding is the tensor core's, not IEEE fma: tolerance
  *          parity (membrane 1e-5, spike flips <= 1e-4), not bit parity.
+ *          Tested against a float64 band (same propagation as FAST) whose
+ *          per-step bound, in threshold units, is
+ *            e_t = (A_t rw + rb) / dom + c_acc 2^-24 (A_t |s| + |b| + |u|) / 2
+ *          with A_t = sum |q| x, dom the domain scale below, rw / rb the
+ *          exact error of the fp16 weight / bias pieces (at least 2^-25 per
+ *          unit of |q| once a piece is an fp16 subnormal) and c_acc = 10: one
+ *          truncation of the fp32 result per MMA, 5 MMAs.  Measured on a
+ *          B200: the accumulation error per step is <= 2.96 * 2^-24 M, and the
+ *          accumulation truncates -- with bias 1 and no input the membrane
+ *          stays at 1 - 2^-24 from step 24 on and never fires, where the
+ *          reference rounds 1 - 2^-25 up to 1.0 and fires at step 25.
  *          Envelope: all 128 channels share one power-of-two domain scale,
  *          fitted to the largest 63.5 * |scale| or |bias| / 2 (fully pruned
  *          channels included).  A channel ~100x the others (all weights
  *          pruned, running var 0) stays inside both bars; with one channel
- *          2^16 or 2^20 times the others the flip bar still holds but some
- *          membranes miss 1e-5 (up to 2.3e-4 relative, no flipped spike,
- *          measured on a B200).  Use EXACT or FAST for such checkpoints. */
+ *          2^16 or 2^20 times the others the other channels' lo weight
+ *          pieces become fp16 subnormals: membranes then miss 1e-5 by up to
+ *          2.3e-4 relative (B200), which the band's 2^-25 floor accounts for
+ *          (measured at 0.56 and 0.90 of delta_T), and the flip bar holds.
+ *          Use EXACT or FAST for such checkpoints. */
 #define SNNQP_LIF_TENSOR 2
 
 /* SpikingBlock(QuantConv 3x3 pad 1, BatchNorm, multi_step_LIF) over T steps
