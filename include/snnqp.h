@@ -196,7 +196,18 @@ typedef struct snnqp_block_params {
  * by the 2x2 max-pool.
  *   x       uint8 [T,B,H,W,Cin] via strides (event counts or {0,1} spikes)
  *   att     NULL, or fp32 per-(t,b,cin) multiplier: input = att * x
- *           (TCJA output y = x_seq * att, models.py:97)
+ *           (TCJA output y = x_seq * att, models.py:97).  With att, x holds
+ *           spikes: any non-zero x byte is a spike (input = att), on every
+ *           implementation.  tcgen05 (SNNQP_IMPL_TCGEN05 / AUTO): att in [0, 1]
+ *           as 24-bit fixed point, round(att 2^24) half to even clamped to
+ *           0xFFFFFF (1.0 reads as 1 - 2^-24), three exact byte-plane
+ *           contractions S2, S1, S0 recombined as fma((float)S2, 65536,
+ *           fma((float)S1, 256, (float)S0)) * 2^-24: |acc - sum att x q| <=
+ *           sum |q| 2^-25 (2^-24 where clamped) + 5 2^-24 M, M = 2^-24 (2^16 |S2|
+ *           + 2^8 |S1| + |S0|).  SIMT: one sequential fp32 fma chain per output
+ *           (kh, kw, channel ascending; dense: k ascending).  Both are bit-exact
+ *           to an emulation (tests/attref.py), which a float64 LIF band checks
+ *           (tests/test_gpu_attention_path.py).
  *   wq      blob from snnqp_pack_conv3x3 (Cin==128) or snnqp_pack_conv1 (Cin==2)
  *   scale/bias fp32 [Cout] from snnqp_fold_affine
  *   spikes  uint8 [T,B,H',W',Cout] via strides, H' = H/2 if pool else H

@@ -67,11 +67,9 @@ k_conv3x3_simt(const snnqp_block_params p, const uint8_t *__restrict__ x,
             if (!ATT && xw == 0u) continue;   // warp-uniform: same pixel for the whole warp
             float xs[4];
             if (ATT) {
+              // with att a non-zero x byte is a spike (input = att), as in the tcgen05 byte-plane expanders
 #pragma unroll
-              for (int j = 0; j < 4; ++j) {
-                const uint32_t sv = (xw >> (8 * j)) & 0xffu;
-                xs[j] = __fmul_rn(__ldg(ab + c4 * 4 + j), (float)sv);
-              }
+              for (int j = 0; j < 4; ++j) xs[j] = ((xw >> (8 * j)) & 0xffu) ? __ldg(ab + c4 * 4 + j) : 0.0f;
             }
 #pragma unroll
             for (int dy = 0; dy < 2; ++dy) {
@@ -259,7 +257,7 @@ k_dense_simt(const snnqp_block_params p, int k_pad, const uint8_t *__restrict__ 
         float a = 0.f;
         if (b < p.B && k < K)
           a = att[(int64_t)t * p.att_stride_t + (int64_t)b * p.att_stride_b + (k % p.att_mod)];
-        sxf[d] = __fmul_rn(a, (float)v);
+        sxf[d] = v ? a : 0.0f;            // with att a non-zero x byte is a spike (input = att)
       }
     }
     __syncthreads();

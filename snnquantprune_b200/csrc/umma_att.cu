@@ -4,13 +4,24 @@
 // models.py:200-216), plus the binary dense2 (models.py:231-246).
 //
 // att is taken as 24-bit fixed point, att ~= (b2*2^16 + b1*2^8 + b0) * 2^-24
-// with u8 bytes b_i (absolute error <= 2^-25), so that
+// with u8 bytes b_i, so that
 //     sum_k att_k s_k q_k = 2^-24 * (2^16 * S2 + 2^8 * S1 + S0),  S_i = sum_k (s_k ? b_i,k : 0) * q_k
 // and each S_i is an EXACT u8 x s8 -> s32 tensor-core contraction over the same
 // packed weights as the binary layers.  "Expander" warps build the three byte
-// planes (spike mask AND attention byte) straight into the swizzled MMA operand
-// layout; the epilogue recombines the three accumulators in fp32.  Error vs the
-// fp32/fp64 evaluation is ~1e-7 in membrane units (tolerance 1e-5).
+// planes (spike mask AND attention byte; any non-zero x byte is a spike) straight
+// into the swizzled MMA operand layout; the epilogue recombines the three
+// accumulators in fp32.  The arithmetic is deterministic and exact but for:
+//  * ptx::att_fix24: round(att * 2^24) half to even, clamped to 0xFFFFFF, so
+//    |att - fix * 2^-24| <= 2^-25, and 2^-24 for att = 1.0 (read as 1 - 2^-24);
+//  * ptx::att_combine: f1 = fma((float)S1, 256, (float)S0), then
+//    f = fma((float)S2, 65536, f1), then the exact * 2^-24 -- five roundings,
+//    each only once a value passes 2^24, each <= 2^-24 M with
+//    M = 2^-24 (2^16 |S2| + 2^8 |S1| + |S0|).
+// So |acc - sum att s q| <= sum_k s_k |q_k| 2^-25 (2^-24 where clamped) + 5 * 2^-24 M.
+// tests/test_gpu_attention_path.py holds both kernels bit-exact to a numpy
+// emulation of exactly these steps (tests/attref.py) and checks a float64 band
+// on that emulation (T = 20, sigmoid-shaped att: ~1e-5 of the conv5
+// neuron-steps undecided, none in dense1).
 //
 //  * k_conv_att_umma : 3x3 conv on 8-wide images (conv5), flat-shift implicit
 //    GEMM exactly as umma_conv.cu, three accumulators per buffer.
