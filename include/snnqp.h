@@ -336,6 +336,32 @@ int snnqp_events_to_frames(const int32_t *addrs, const int64_t *offsets, int B,
                            int64_t max_events_per_sample, void *frames,
                            int out_int32, uint64_t *n_saturated, void *stream);
 
+/* Packed event words: the host -> device wire format of event input.  One word
+ * per event, in time order:
+ *   SNNQP_EVENTS_U16  uint16 w: x = w & 0x7F, y = (w >> 7) & 0x7F, p = w >> 15;
+ *                     bit 14 is zero.  Every x, y < 128 (a 128 x 128 sensor).
+ *   SNNQP_EVENTS_U32  uint32 w: x = w & 0x7FFF, y = (w >> 15) & 0x7FFF,
+ *                     p = w >> 31; bit 30 is zero.  Every x, y < 32768.
+ * p is the polarity bit (p != 0 of the record).  Encoder on the host:
+ * snnquantprune_b200/input_pipeline.py (encode_events). */
+#define SNNQP_EVENTS_U16 1
+#define SNNQP_EVENTS_U32 2
+
+/* snnqp_events_to_frames on packed event words (event_format = SNNQP_EVENTS_*):
+ * same split, cells, flat-position rule, saturation and counter choice.  Sample
+ * b's events are events[offsets[b] - event_base, offsets[b+1] - event_base):
+ * a batch is encoded once, and any sample range [b0, b1) is then the words
+ * [offsets[b0], offsets[b1]) plus offsets[b0 .. b1], shipped as they are with
+ * event_base = offsets[b0].  events and frames must be 16-byte aligned (the
+ * words are read as 16-byte vectors; group bounds may fall at any word). */
+int snnqp_events_to_frames_packed(const void *events, int event_format,
+                                  const int64_t *offsets, int64_t event_base,
+                                  int B, int T, int sensor_wh,
+                                  int resolution_scale,
+                                  int64_t max_events_per_sample, void *frames,
+                                  int out_int32, uint64_t *n_saturated,
+                                  void *stream);
+
 /* Activation-density numerators (examples/tcja/models.py:128-142 sows
  * sum(x != 0) over (H,W,C) per (t,b) slice / slice size, then max and mean):
  * counts[i] = number of non-zero bytes of slice i (slice_bytes long, slices

@@ -15,6 +15,7 @@ ABI_VERSION = 3          # include/snnqp.h SNNQP_ABI_VERSION (block params carry
 IMPL_AUTO, IMPL_SIMT, IMPL_TCGEN05 = 0, 1, 2
 SPIKES_U8, SPIKES_BITS = 0, 1
 LIF_EXACT, LIF_FAST, LIF_TENSOR = 0, 1, 2
+EVENTS_U16, EVENTS_U32 = 1, 2     # packed event words (snnqp_events_to_frames_packed)
 
 
 class SnnqpError(RuntimeError):
@@ -64,6 +65,7 @@ SIGNATURES = {
     "snnqp_vote_fwd": (_i, [_vp, _i, _i, _i, _i, _i64, _i64, _vp, _vp]),
     "snnqp_eval_metrics": (_i, [_vp, _vp, _i, _i, _vp, _vp]),
     "snnqp_events_to_frames": (_i, [_vp, _vp, _i, _i, _i, _i, _i64, _vp, _i, _vp, _vp]),
+    "snnqp_events_to_frames_packed": (_i, [_vp, _i, _vp, _i64, _i, _i, _i, _i, _i64, _vp, _i, _vp, _vp]),
     "snnqp_slice_nonzeros": (_i, [_vp, _i, _i64, _i64, _vp, _vp]),
     "snnqp_slice_popcount": (_i, [_vp, _i, _i64, _i64, _vp, _vp]),
     "snnqp_spiking_head_fwd": (_i, [_BP, _vp, _vp, _vp, _vp, _vp, _BP, _vp, _vp, _vp, _vp, _vp, _vp]),

@@ -5,43 +5,91 @@
 //   cut into T consecutive groups of di = N / T events (the last group takes the remainder), and each
 //   group is histogrammed into a (wh, wh, 2) frame: cell = ((y / rs) * wh + x / rs) * 2 + (p != 0).
 //   One CTA per (sample, frame): the whole histogram lives in shared memory (64 KB at wh = 128 with 16-bit
-//   counters -- three frames in flight per SM; 128 KB with 32-bit ones), events are read once with coalesced 12-byte records, all atomics are shared-memory
+//   counters -- three frames in flight per SM; 128 KB with 32-bit ones), events are read once (coalesced 12-byte
+//   int32 records, or 2- / 4-byte packed words in 16-byte vectors: snnqp_events_to_frames_packed), all atomics are shared-memory
 //   atomics, and the frame leaves as one pass of 128-bit stores in the hot path's own input layout
 //   [B][T][H][W][2] (uint8, saturating, saturated cells counted; or exact int32).
 //
 // k_slice_nonzeros: number of non-zero bytes of each (t, b) slice of a u8 activation tensor -- the
 //   numerator of the densities the reference sows (examples/tcja/models.py:128-142: sum(x != 0) over
 //   (H, W, C) per (t, b), then max / mean on the host).
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace snnqp {
 namespace {
 
+// Event record decoders.  I32x3: int32 (x, y, p) triples.  U16 / U32: one packed word per event (include/snnqp.h,
+// SNNQP_EVENTS_U16 / _U32), read as 16-byte vectors over the aligned interior of each group.
+struct EvI32x3 {};
+struct EvU16 {
+  using Word = uint16_t;
+  __device__ static void decode(uint32_t w, int &x, int &y, int &p) { x = w & 0x7F; y = (w >> 7) & 0x7F; p = w >> 15; }
+};
+struct EvU32 {
+  using Word = uint32_t;
+  __device__ static void decode(uint32_t w, int &x, int &y, int &p) { x = w & 0x7FFF; y = (w >> 15) & 0x7FFF; p = w >> 31; }
+};
+
 // PACKED: the two polarity counters of a pixel share one 32-bit word (16 bits each) -- 64 KB per frame at
 // wh = 128, three CTAs per SM; exact while a frame holds < 65536 events (the launcher checks the caller's bound).
 // !PACKED: one int32 per cell (128 KB, one CTA per SM), exact for any count.
-template <typename OutT, bool PACKED>
+// Sample b's events are events[offsets[b] - event_base, offsets[b + 1] - event_base).
+template <typename Dec, typename OutT, bool PACKED>
 __global__ void __launch_bounds__(512, PACKED ? 3 : 1)
-k_events_to_frames(const int32_t *__restrict__ addrs, const int64_t *__restrict__ offsets, int T, int wh, int rs,
-                   OutT *__restrict__ frames, unsigned long long *__restrict__ n_saturated) {
+k_events_to_frames(const void *__restrict__ events, const int64_t *__restrict__ offsets, int64_t event_base, int T,
+                   int wh, int rs, OutT *__restrict__ frames, unsigned long long *__restrict__ n_saturated) {
   extern __shared__ int hist[];
   const int b = blockIdx.x / T, t = blockIdx.x % T;
   const int pixels = wh * wh;
   const int words = PACKED ? pixels : 2 * pixels;
   for (int i = threadIdx.x; i < words / 4; i += blockDim.x) reinterpret_cast<int4 *>(hist)[i] = make_int4(0, 0, 0, 0);
   __syncthreads();
-  const int64_t e0 = offsets[b], n = offsets[b + 1] - e0;
+  const int64_t e0 = offsets[b] - event_base, n = offsets[b + 1] - offsets[b];
   const int64_t di = n / T;
   const int64_t lo = e0 + (int64_t)t * di, hi = (t < T - 1) ? lo + di : e0 + n;
-  // 12-byte records: three coalesced word streams
-  for (int64_t e = lo + threadIdx.x; e < hi; e += blockDim.x) {
-    const int x = __ldg(addrs + 3 * e) / rs, y = __ldg(addrs + 3 * e + 1) / rs, p = __ldg(addrs + 3 * e + 2);
-    // the reference histograms the FLAT position y*wh + x (input_pipeline.py:196-199): an x beyond the row
-    // lands in the next row, exactly as there; only positions outside the frame are dropped
+  // the reference histograms the FLAT position y*wh + x (input_pipeline.py:196-199): an x beyond the row
+  // lands in the next row, exactly as there; only positions outside the frame are dropped
+  auto count = [&](int x, int y, int p) {
     const int64_t pos = (int64_t)y * wh + x;
     if (pos >= 0 && pos < (int64_t)pixels) {
       if constexpr (PACKED) atomicAdd(hist + pos, p != 0 ? 0x10000 : 1);
       else atomicAdd(hist + (pos << 1) + (p != 0 ? 1 : 0), 1);
+    }
+  };
+  if constexpr (std::is_same<Dec, EvI32x3>::value) {
+    // 12-byte records: three coalesced word streams
+    const int32_t *addrs = static_cast<const int32_t *>(events);
+    for (int64_t e = lo + threadIdx.x; e < hi; e += blockDim.x)
+      count(__ldg(addrs + 3 * e) / rs, __ldg(addrs + 3 * e + 1) / rs, __ldg(addrs + 3 * e + 2));
+  } else {
+    using W = typename Dec::Word;
+    constexpr int V = 16 / sizeof(W);                   // words per 16-byte vector (events is 16-byte aligned)
+    const W *ev = static_cast<const W *>(events);
+    auto one = [&](uint32_t w) {
+      int x, y, p;
+      Dec::decode(w, x, y, p);
+      count(x / rs, y / rs, p);
+    };
+    // [v0, v1): the whole vectors inside [lo, hi); the head [lo, V v0) and tail [V v1, hi) go word by word
+    const int64_t v0 = (lo + V - 1) / V, v1 = hi / V > v0 ? hi / V : v0;
+    const int64_t head_end = V * v0 < hi ? V * v0 : hi;
+    for (int64_t e = lo + threadIdx.x; e < head_end; e += blockDim.x) one(__ldg(ev + e));
+    for (int64_t e = (V * v1 > head_end ? V * v1 : head_end) + threadIdx.x; e < hi; e += blockDim.x) one(__ldg(ev + e));
+    const uint4 *vec = reinterpret_cast<const uint4 *>(ev);
+    for (int64_t v = v0 + threadIdx.x; v < v1; v += blockDim.x) {
+      const uint4 q = __ldg(vec + v);
+      const uint32_t q4[4] = {q.x, q.y, q.z, q.w};
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        if constexpr (sizeof(W) == 2) {
+          one(q4[k] & 0xFFFFu);
+          one(q4[k] >> 16);
+        } else {
+          one(q4[k]);
+        }
+      }
     }
   }
   __syncthreads();
@@ -103,14 +151,40 @@ k_slice_nonzeros(const uint8_t *__restrict__ x, int64_t slice_bytes, int64_t str
 }  // namespace snnqp
 
 namespace snnqp {
-template <typename OutT, bool PACKED>
-static int launch_events(const int32_t *addrs, const int64_t *offsets, int B, int T, int wh, int rs, OutT *frames,
-                         unsigned long long *n_sat, cudaStream_t st) {
+template <typename Dec, typename OutT, bool PACKED>
+static int launch_events(const void *events, const int64_t *offsets, int64_t event_base, int B, int T, int wh, int rs,
+                         OutT *frames, unsigned long long *n_sat, cudaStream_t st) {
   const size_t smem = (size_t)(PACKED ? 1 : 2) * wh * wh * sizeof(int);
-  SNNQP_CUDA(cudaFuncSetAttribute(k_events_to_frames<OutT, PACKED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  k_events_to_frames<OutT, PACKED><<<B * T, 512, smem, st>>>(addrs, offsets, T, wh, rs, frames, n_sat);
+  auto k = k_events_to_frames<Dec, OutT, PACKED>;
+  SNNQP_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k<<<B * T, 512, smem, st>>>(events, offsets, event_base, T, wh, rs, frames, n_sat);
   SNNQP_POST_LAUNCH("k_events_to_frames");
   return SNNQP_OK;
+}
+
+// checks shared by both entry points (events, offsets and frames are non-null), then the launch
+template <typename Dec>
+static int events_to_frames(const char *fn, const void *events, const int64_t *offsets, int64_t event_base, int B,
+                            int T, int sensor_wh, int resolution_scale, int64_t max_events_per_sample, void *frames,
+                            int out_int32, uint64_t *n_saturated, cudaStream_t st) {
+  if (B <= 0 || T <= 0 || sensor_wh <= 0 || resolution_scale <= 0) return invalid("%s: B, T, wh, scale must be > 0", fn);
+  const int wh = sensor_wh / resolution_scale;
+  if (wh <= 0 || (2 * wh * wh) % 16) return invalid("%s: 2*wh*wh must be a multiple of 16 (wh = %d)", fn, wh);
+  if ((size_t)2 * wh * wh * sizeof(int) > 200 * 1024)
+    return unsupported("%s: frame of %d x %d x 2 does not fit the shared-memory histogram", fn, wh, wh);
+  if (reinterpret_cast<uintptr_t>(frames) & 15) return invalid("%s: frames must be 16-byte aligned", fn);
+  // a frame holds at most N/T + (T-1) events: 16-bit counters are exact below 65536
+  const bool packed = max_events_per_sample > 0 && max_events_per_sample / T + T < 65536;
+  const int rs = resolution_scale;
+  unsigned long long *ns = reinterpret_cast<unsigned long long *>(n_saturated);
+  if (out_int32) {
+    int32_t *f = static_cast<int32_t *>(frames);
+    return packed ? launch_events<Dec, int32_t, true>(events, offsets, event_base, B, T, wh, rs, f, nullptr, st)
+                  : launch_events<Dec, int32_t, false>(events, offsets, event_base, B, T, wh, rs, f, nullptr, st);
+  }
+  uint8_t *f = static_cast<uint8_t *>(frames);
+  return packed ? launch_events<Dec, uint8_t, true>(events, offsets, event_base, B, T, wh, rs, f, ns, st)
+                : launch_events<Dec, uint8_t, false>(events, offsets, event_base, B, T, wh, rs, f, ns, st);
 }
 }  // namespace snnqp
 
@@ -119,25 +193,29 @@ extern "C" int snnqp_events_to_frames(const int32_t *addrs, const int64_t *offse
                                       uint64_t *n_saturated, void *stream_) {
   using namespace snnqp;
   if (int r = require_device()) return r;
-  cudaStream_t st = static_cast<cudaStream_t>(stream_);
   if (!addrs || !offsets || !frames) return invalid("snnqp_events_to_frames: null pointer");
-  if (B <= 0 || T <= 0 || sensor_wh <= 0 || resolution_scale <= 0) return invalid("snnqp_events_to_frames: B, T, wh, scale must be > 0");
-  const int wh = sensor_wh / resolution_scale;
-  if (wh <= 0 || (2 * wh * wh) % 16) return invalid("snnqp_events_to_frames: 2*wh*wh must be a multiple of 16 (wh = %d)", wh);
-  if ((size_t)2 * wh * wh * sizeof(int) > 200 * 1024)
-    return unsupported("snnqp_events_to_frames: frame of %d x %d x 2 does not fit the shared-memory histogram", wh, wh);
-  if (reinterpret_cast<uintptr_t>(frames) & 15) return invalid("snnqp_events_to_frames: frames must be 16-byte aligned");
-  // a frame holds at most N/T + (T-1) events: 16-bit counters are exact below 65536
-  const bool packed = max_events_per_sample > 0 && max_events_per_sample / T + T < 65536;
-  unsigned long long *ns = reinterpret_cast<unsigned long long *>(n_saturated);
-  if (out_int32) {
-    int32_t *f = static_cast<int32_t *>(frames);
-    return packed ? launch_events<int32_t, true>(addrs, offsets, B, T, wh, resolution_scale, f, nullptr, st)
-                  : launch_events<int32_t, false>(addrs, offsets, B, T, wh, resolution_scale, f, nullptr, st);
-  }
-  uint8_t *f = static_cast<uint8_t *>(frames);
-  return packed ? launch_events<uint8_t, true>(addrs, offsets, B, T, wh, resolution_scale, f, ns, st)
-                : launch_events<uint8_t, false>(addrs, offsets, B, T, wh, resolution_scale, f, ns, st);
+  return events_to_frames<EvI32x3>("snnqp_events_to_frames", addrs, offsets, 0, B, T, sensor_wh, resolution_scale,
+                                   max_events_per_sample, frames, out_int32, n_saturated,
+                                   static_cast<cudaStream_t>(stream_));
+}
+
+extern "C" int snnqp_events_to_frames_packed(const void *events, int event_format, const int64_t *offsets,
+                                             int64_t event_base, int B, int T, int sensor_wh, int resolution_scale,
+                                             int64_t max_events_per_sample, void *frames, int out_int32,
+                                             uint64_t *n_saturated, void *stream_) {
+  using namespace snnqp;
+  static const char fn[] = "snnqp_events_to_frames_packed";
+  if (int r = require_device()) return r;
+  if (!events || !offsets || !frames) return invalid("%s: null pointer", fn);
+  if (reinterpret_cast<uintptr_t>(events) & 15) return invalid("%s: events must be 16-byte aligned", fn);
+  cudaStream_t st = static_cast<cudaStream_t>(stream_);
+  if (event_format == SNNQP_EVENTS_U16)
+    return events_to_frames<EvU16>(fn, events, offsets, event_base, B, T, sensor_wh, resolution_scale,
+                                   max_events_per_sample, frames, out_int32, n_saturated, st);
+  if (event_format == SNNQP_EVENTS_U32)
+    return events_to_frames<EvU32>(fn, events, offsets, event_base, B, T, sensor_wh, resolution_scale,
+                                   max_events_per_sample, frames, out_int32, n_saturated, st);
+  return invalid("%s: event_format = %d (SNNQP_EVENTS_U16 or SNNQP_EVENTS_U32)", fn, event_format);
 }
 
 static int slice_count(const uint8_t *x, int n_slices, int64_t slice_bytes, int64_t stride_slice, int32_t *counts,

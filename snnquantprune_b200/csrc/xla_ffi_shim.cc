@@ -131,6 +131,28 @@ XLA_FFI_DEFINE_HANDLER_SYMBOL(SnnqpEventsToFrames, EventsToFramesImpl,
                                   .Attr<int32_t>("resolution_scale")
                                   .Attr<int64_t>("max_events_per_sample"));
 
+// packed event words (SNNQP_EVENTS_U16 / _U32, include/snnqp.h) -> frames: events is the words' raw bytes (N * 2 or
+// N * 4 uint8, e.g. lax.bitcast_convert_type of the uint16 / uint32 words), offsets (B+1) int64 relative to event_base
+static ffi::Error EventsToFramesPackedImpl(cudaStream_t stream, ffi::Buffer<ffi::U8> events, ffi::Buffer<ffi::S64> offsets,
+                                           ffi::ResultBuffer<ffi::U8> frames, int32_t event_format, int32_t sensor_wh,
+                                           int32_t resolution_scale, int64_t max_events_per_sample, int64_t event_base) {
+  auto f = frames->dimensions();                // (B, T, wh, wh, 2)
+  return Status(snnqp_events_to_frames_packed(events.typed_data(), event_format, offsets.typed_data(), event_base,
+                                              (int)f[0], (int)f[1], sensor_wh, resolution_scale, max_events_per_sample,
+                                              frames->typed_data(), 0, nullptr, stream));
+}
+XLA_FFI_DEFINE_HANDLER_SYMBOL(SnnqpEventsToFramesPacked, EventsToFramesPackedImpl,
+                              ffi::Ffi::Bind()
+                                  .Ctx<ffi::PlatformStream<cudaStream_t>>()
+                                  .Arg<ffi::Buffer<ffi::U8>>()
+                                  .Arg<ffi::Buffer<ffi::S64>>()
+                                  .Ret<ffi::Buffer<ffi::U8>>()
+                                  .Attr<int32_t>("event_format")
+                                  .Attr<int32_t>("sensor_wh")
+                                  .Attr<int32_t>("resolution_scale")
+                                  .Attr<int64_t>("max_events_per_sample")
+                                  .Attr<int64_t>("event_base"));
+
 // ---- the att-weighted / counting variants that wire conv4 -> TCJA -> conv5 -> dense1 (examples/tcja/models.py:
 // 151-246): the binding a maintainer adds inside SpikingBlock.__call__ (spiking_learning.py:454-462) ---------------
 static void FillConv(snnqp_block_params &p, const std::vector<int64_t> &d, int32_t cout, int32_t pool, float tau,

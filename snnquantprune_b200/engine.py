@@ -460,6 +460,70 @@ class CextNetEngine:
       return out_host
     return logits
 
+  def forward_host_events(self, eb, resolution_scale: int = 1, out_host: Optional[torch.Tensor] = None,
+                          n_saturated: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """End-to-end call from HOST memory on event recordings (``input_pipeline.EventBatch``: one packed word per event,
+    what the reference's loader holds before it integrates frames).  Per chunk: two pinned-memory copies (words,
+    offsets) on the side stream, ``snnqp_events_to_frames_packed`` into the staging frame buffer, then the same head /
+    tail launches as :meth:`forward`; copies of chunk k+1 overlap the conv1-3 kernels of chunk k.  The frames are
+    uint8, saturating at 255: ``n_saturated`` (device int64 scalar), if given, accumulates the saturated cells (no
+    host sync)."""
+    from .input_pipeline import events_to_frames_packed
+    pk = self.pk
+    if eb.events.is_cuda:
+      raise ValueError("forward_host_events takes the (pinned) host tensors of an EventBatch")
+    if int(resolution_scale) != resolution_scale or resolution_scale < 1 or eb.sensor_wh // resolution_scale != pk.H:
+      raise ValueError(f"sensor {eb.sensor_wh} // resolution_scale {resolution_scale} != H = {pk.H}")
+    B = eb.shape[0]
+    Bc = min(self.chunk, B)
+    ws = self._workspace(B, Bc)
+    chunks = self.host_chunks(B)
+    o = eb.offsets.numpy()
+    emax = max(int(o[b0 + n] - o[b0]) for b0, n in chunks)
+    if "stage" not in ws:
+      ws["stage"] = torch.empty((2, Bc, pk.T, pk.H, pk.H, 2), device=self.device, dtype=torch.uint8)
+    ev = ws.get("ev")
+    if ev is None or ev[0][0].dtype != eb.events.dtype or ev[0][0].numel() < emax:
+      # sized to the largest chunk; safe to replace: the side stream waits for the current stream before its first copy
+      ws["ev"] = ev = [(torch.empty(max(emax, 1), device=self.device, dtype=eb.events.dtype),
+                        torch.empty(Bc + 1, device=self.device, dtype=torch.int64)) for _ in range(2)]
+    if n_saturated is None:                             # a scratch counter: no fill launch per chunk
+      if "ev_sat" not in ws:
+        ws["ev_sat"] = torch.zeros((), device=self.device, dtype=torch.int64)
+      n_saturated = ws["ev_sat"]
+    if not hasattr(self, "_copy_stream"):
+      self._copy_stream = torch.cuda.Stream(device=self.device)
+    cur = torch.cuda.current_stream(self.device)
+    logits = torch.empty((B, pk.num_classes), device=self.device, dtype=torch.float32)
+    self._copy_stream.wait_stream(cur)
+    done = []
+    pipe = _HeadPipe(self, ws)
+    for i, (b0, n) in enumerate(chunks):
+      words, offs, base = eb.chunk(b0, b0 + n)
+      dev, doff = ev[i & 1]
+      buf = ws["stage"][i & 1][:n]
+      if i >= 2:
+        self._copy_stream.wait_event(done[i - 2])       # staging buffers free again
+      with torch.cuda.stream(self._copy_stream):
+        dev[:words.numel()].copy_(words, non_blocking=True)
+        doff[:n + 1].copy_(offs, non_blocking=True)
+        ready = torch.cuda.Event()
+        ready.record(self._copy_stream)
+      cur.wait_event(ready)
+      events_to_frames_packed(dev, doff[:n + 1], eb.format, pk.T, eb.sensor_wh, resolution_scale, out=buf,
+                              max_events_per_sample=eb.max_events_per_sample, event_base=base,
+                              n_saturated=n_saturated)
+      pipe.push(buf, b0, n)
+      e = torch.cuda.Event()
+      e.record(cur)
+      done.append(e)
+    pipe.finish()
+    self._tail(B, ws, logits)
+    if out_host is not None:
+      out_host.copy_(logits, non_blocking=True)
+      return out_host
+    return logits
+
   def forward_graph(self, frames: torch.Tensor) -> torch.Tensor:
     """Same as :meth:`forward`, replayed from a CUDA graph captured on the first
     call for this (buffer, batch) -- removes the per-launch host overhead.  The

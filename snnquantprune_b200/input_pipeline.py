@@ -4,7 +4,14 @@ entry-point name and argument meaning
 ``split_by == "number"`` only -- the reference raises NotImplementedError for
 "time" too), on the GPU: the frames are produced directly in HBM in the hot
 path's input layout (B,T,H,W,2) uint8, so real event streams never touch a CPU
-histogram.  No CPU fallback."""
+histogram.  No CPU fallback.
+
+Three host -> device wire formats feed the end-to-end host calls of
+``CextNetEngine``: dense uint8 frames (``forward_host``), zero-suppressed frames
+(``ZsfBatch``, ``forward_host_zsf``) and packed event words (``EventBatch``,
+``forward_host_events``): the recordings as the reference's loader holds them,
+one 16- or 32-bit word per event, integrated into frames on the GPU chunk by
+chunk."""
 from __future__ import annotations
 
 from typing import Optional, Sequence, Tuple
@@ -158,3 +165,107 @@ def zsf_expand(bitmap: torch.Tensor, block_off: torch.Tensor, values: torch.Tens
                                                 int(value_base), int(n_blocks), int(value_bits), _lib.ptr(out),
                                                 _lib.stream()))
   return out
+
+
+# ---- packed events: the event-list wire format of the end-to-end path -------------------------------------------
+class EventBatch:
+  """A batch of event recordings as packed words (``snnqp_events_to_frames_packed``, include/snnqp.h): ``events`` holds
+  one word per event, all samples back to back in time order (int16 carrying the SNNQP_EVENTS_U16 bits, or int32
+  carrying the SNNQP_EVENTS_U32 bits); ``offsets`` int64 [B+1] index sample b's words as
+  ``events[offsets[b]:offsets[b+1]]``.  Tensors are pinned CPU tensors when CUDA is available.  ``eb[lo:hi]`` is a view
+  of samples [lo, hi) (it shares ``events``); ``chunk(b0, b1)`` is what one host -> device copy of that range ships."""
+
+  def __init__(self, events: torch.Tensor, offsets: torch.Tensor, format: int, sensor_wh: int,
+               max_events_per_sample: int):
+    self.events, self.offsets = events, offsets
+    self.format = int(format)
+    self.sensor_wh = int(sensor_wh)
+    self.max_events_per_sample = int(max_events_per_sample)        # an upper bound of every sample's event count
+
+  @property
+  def shape(self):
+    return (self.offsets.numel() - 1,)
+
+  @property
+  def nbytes(self) -> int:
+    """Wire bytes of the batch: its words plus its offsets."""
+    o0, o1 = int(self.offsets[0]), int(self.offsets[-1])
+    return (o1 - o0) * self.events.element_size() + self.offsets.numel() * 8
+
+  def __len__(self):
+    return self.shape[0]
+
+  def __getitem__(self, key):
+    if not isinstance(key, slice) or key.step not in (None, 1):
+      raise TypeError("EventBatch supports contiguous slices only")
+    lo, hi, _ = key.indices(self.shape[0])
+    hi = max(hi, lo)
+    return EventBatch(self.events, self.offsets[lo:hi + 1], self.format, self.sensor_wh, self.max_events_per_sample)
+
+  def chunk(self, b0: int, b1: int):
+    """(events slice, offsets slice, event_base) for samples [b0, b1): the words of those samples, their offsets
+    ``offsets[b0:b1+1]`` unchanged, and ``event_base = offsets[b0]``."""
+    e0, e1 = int(self.offsets[b0]), int(self.offsets[b1])
+    return self.events[e0:e1], self.offsets[b0:b1 + 1], e0
+
+
+def encode_events(samples: Sequence[np.ndarray], sensor_wh: int) -> EventBatch:
+  """Host-side encoder (data-loader side, numpy): list of (N_b, 3) integer (x, y, p) arrays in time order ->
+  :class:`EventBatch`.  SNNQP_EVENTS_U16 when every x, y < 128, else SNNQP_EVENTS_U32 (every x, y < 2^15); p != 0
+  becomes the polarity bit.  No event is dropped: every event counts toward the split of its sample, and an x beyond
+  the sensor row is histogrammed at its flat position, as in ``events_to_frames``."""
+  sizes = np.array([int(np.shape(a)[0]) for a in samples], np.int64)
+  off = np.zeros(len(samples) + 1, np.int64)
+  off[1:] = np.cumsum(sizes)
+  flat = np.concatenate([np.asarray(a).reshape(-1, 3) for a in samples], 0) if off[-1] else np.zeros((0, 3), np.int64)
+  if flat.dtype.kind not in "iu":
+    raise ValueError("encode_events takes integer (x, y, p) records")
+  xy = flat[:, :2]
+  lo, hi = (int(xy.min()), int(xy.max())) if xy.size else (0, 0)
+  if lo < 0 or hi >= 2 ** 15:
+    bad = np.flatnonzero(((xy < 0) | (xy >= 2 ** 15)).any(1))
+    b = int(np.searchsorted(off, bad[0], side="right") - 1)
+    raise ValueError(f"encode_events: sample {b} has an event at (x, y) = {tuple(int(v) for v in xy[bad[0]])}, "
+                     "outside [0, 32768); integrate such recordings with concat_events + events_to_frames")
+  x, y = xy[:, 0].astype(np.uint32), xy[:, 1].astype(np.uint32)
+  p = (flat[:, 2] != 0).astype(np.uint32)
+  if hi < 128:
+    fmt = _lib.EVENTS_U16
+    words = (x | (y << 7) | (p << 15)).astype(np.uint16).view(np.int16)
+  else:
+    fmt = _lib.EVENTS_U32
+    words = (x | (y << 15) | (p << 31)).view(np.int32)
+  ev, offsets = torch.as_tensor(np.ascontiguousarray(words)), torch.as_tensor(off)
+  if torch.cuda.is_available():
+    ev, offsets = ev.pin_memory(), offsets.pin_memory()
+  return EventBatch(ev, offsets, fmt, sensor_wh, int(sizes.max(initial=0)))
+
+
+def events_to_frames_packed(events: torch.Tensor, offsets: torch.Tensor, event_format: int, num_frames: int, wh: int,
+                            resolution_scale: int = 1, exact_int32: bool = False, out: Optional[torch.Tensor] = None,
+                            max_events_per_sample: int = 0, event_base: int = 0,
+                            n_saturated: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+  """:func:`events_to_frames` on packed event words (device tensors: ``events`` int16 for SNNQP_EVENTS_U16 or int32
+  for SNNQP_EVENTS_U32, 16-byte aligned; ``offsets`` int64 [B+1], sample b's words at ``offsets[b] - event_base``).
+  Returns (frames, n_saturated); a given ``n_saturated`` (device int64 scalar) is accumulated into, no host sync."""
+  if int(resolution_scale) != resolution_scale or resolution_scale < 1:
+    raise NotImplementedError("resolution_scale must be a positive integer")
+  want = {_lib.EVENTS_U16: torch.int16, _lib.EVENTS_U32: torch.int32}.get(int(event_format))
+  if want is None or events.dtype != want or offsets.dtype != torch.int64:
+    raise ValueError("events must be int16 (EVENTS_U16) or int32 (EVENTS_U32) words and offsets int64 (B+1,)")
+  B = offsets.numel() - 1
+  whs = int(wh // resolution_scale)
+  dt = torch.int32 if exact_int32 else torch.uint8
+  if out is None:
+    out = torch.empty((B, num_frames, whs, whs, 2), device=events.device, dtype=dt)
+  if n_saturated is None:
+    n_saturated = torch.zeros((), device=events.device, dtype=torch.int64)
+  elif not n_saturated.is_cuda or n_saturated.dtype != torch.int64 or n_saturated.numel() != 1:
+    raise ValueError("n_saturated must be a device int64 scalar")
+  if B == 0:
+    return out, n_saturated
+  _lib.check(_lib.lib().snnqp_events_to_frames_packed(
+      _lib.ptr(events), int(event_format), _lib.ptr(offsets), int(event_base), B, num_frames, int(wh),
+      int(resolution_scale), int(max_events_per_sample), _lib.ptr(out), 1 if exact_int32 else 0,
+      _lib.ptr(n_saturated), _lib.stream()))
+  return out, n_saturated

@@ -176,6 +176,24 @@ def make_frames(B: int, T: int = 20, H: int = 128, W: int = 128, seed: int = 0,
   return np.minimum(rng.poisson(rate, size=(B, T, H, W, 2)), 15).astype(np.uint8)
 
 
+def make_events(B: int, T: int = 20, H: int = 128, seed: int = 0, rate: float = 0.15):
+  """Synthetic event recordings: a list of B int32 (N_b, 3) (x, y, p) arrays, x, y uniform on the H x H sensor, p
+  uniform in {0, 1}.  N_b is uniform within +-25 % of ``rate * T * H * H * 2`` (so each cell of the T frames gets
+  about ``rate`` events, as in :func:`make_frames`), so sizes vary and N_b % T is mostly non-zero.  Drawn from
+  :class:`StableRNG`: identical on every numpy."""
+  rng = StableRNG(seed)
+  mean = int(round(rate * T * H * H * 2))
+  spread = mean // 4
+  sizes = rng.integers(mean - spread, mean + spread + 1, (B,))
+  out = []
+  for n in sizes:
+    n = int(n)
+    xy = rng.integers(0, H, (n, 2))
+    p = rng.integers(0, 2, (n, 1))
+    out.append(np.concatenate([xy, p], 1).astype(np.int32))
+  return out
+
+
 def make_labels(B: int, num_classes: int = 11, seed: int = 3) -> np.ndarray:
   return np.random.default_rng(seed).integers(0, num_classes, size=(B,)).astype(np.int32)
 
