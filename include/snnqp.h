@@ -322,7 +322,9 @@ int64_t snnqp_launch_count(int reset);
  * of all samples back to back in time order, offsets = int64 [B+1] record
  * offsets.  Sample b's events are cut into T groups of N_b / T events (the
  * last takes the remainder); group t is histogrammed into frame (b, t):
- * cell ((y/rs)*wh + x/rs, p != 0), wh = sensor_wh / rs.  frames: [B][T][wh][wh][2]
+ * cell (floor(y/rs)*wh + floor(x/rs), p != 0), wh = sensor_wh / rs (floor, as
+ * the reference's floor-division: a negative coordinate rounds down, so (-1, y)
+ * at rs = 2 is the previous row's last pixel).  frames: [B][T][wh][wh][2]
  * uint8 saturating at 255 (out_int32 == 0; *n_saturated += saturated cells, may
  * be NULL) or exact int32 (out_int32 != 0).  Like the reference, the FLAT
  * position is histogrammed (an x beyond the row lands in the next row); only

@@ -3,7 +3,7 @@
 // k_events_to_frames: DVS events -> event-count frames, "split by number"
 //   (reference examples/input_pipeline.py:142-219, preprocess_data_number): the N events of a sample are
 //   cut into T consecutive groups of di = N / T events (the last group takes the remainder), and each
-//   group is histogrammed into a (wh, wh, 2) frame: cell = ((y / rs) * wh + x / rs) * 2 + (p != 0).
+//   group is histogrammed into a (wh, wh, 2) frame: cell = (floor(y / rs) * wh + floor(x / rs)) * 2 + (p != 0).
 //   One CTA per (sample, frame): the whole histogram lives in shared memory (64 KB at wh = 128 with 16-bit
 //   counters -- three frames in flight per SM; 128 KB with 32-bit ones), events are read once (coalesced 12-byte
 //   int32 records, or 2- / 4-byte packed words in 16-byte vectors: snnqp_events_to_frames_packed), all atomics are shared-memory
@@ -59,10 +59,12 @@ k_events_to_frames(const void *__restrict__ events, const int64_t *__restrict__ 
     }
   };
   if constexpr (std::is_same<Dec, EvI32x3>::value) {
-    // 12-byte records: three coalesced word streams
+    // 12-byte records: three coalesced word streams.  Coordinates may be negative here: floor(v / rs), as the
+    // reference's float floor-division (input_pipeline.py:183-190), not C's truncation toward zero
     const int32_t *addrs = static_cast<const int32_t *>(events);
+    auto floor_div = [rs](int v) { return v >= 0 ? v / rs : -1 - (-1 - v) / rs; };
     for (int64_t e = lo + threadIdx.x; e < hi; e += blockDim.x)
-      count(__ldg(addrs + 3 * e) / rs, __ldg(addrs + 3 * e + 1) / rs, __ldg(addrs + 3 * e + 2));
+      count(floor_div(__ldg(addrs + 3 * e)), floor_div(__ldg(addrs + 3 * e + 1)), __ldg(addrs + 3 * e + 2));
   } else {
     using W = typename Dec::Word;
     constexpr int V = 16 / sizeof(W);                   // words per 16-byte vector (events is 16-byte aligned)
