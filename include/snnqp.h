@@ -40,7 +40,7 @@
 extern "C" {
 #endif
 
-#define SNNQP_ABI_VERSION 3
+#define SNNQP_ABI_VERSION 4
 
 #define SNNQP_OK 0
 #define SNNQP_ERR_INVALID 1      /* bad argument / unsupported shape           */
@@ -232,23 +232,6 @@ int snnqp_spiking_conv3x3_counts_fwd(const snnqp_block_params *p, const uint8_t 
                                      uint8_t *spikes, float *u_final, void *acc_dump,
                                      int32_t *spike_counts, void *stream);
 
-/* Blocks 1 and 2 of CextNet (examples/tcja/models.py:111-147) in ONE persistent
- * kernel, each on its own sample range: block 1 (QuantConv 2 -> 128 channels at
- * HxW, bound by its LIF epilogue's issue slots) and block 2 (128 -> 128 at
- * 64x64, bound by the tensor pipe) share every SM, so the forward of a long
- * batch runs block 1 of chunk k+1 under block 2 of chunk k.  Either half may be
- * absent (p == NULL or B == 0: the first / last launch of a batch).  Operands as
- * in snnqp_spiking_conv3x3_fwd; block 1 takes SNNQP_SPIKES_U8 counts and emits
- * SNNQP_SPIKES_BITS, block 2 takes SNNQP_SPIKES_BITS; both need the standard LIF
- * constants (tau 2, threshold 1, reset 0) and pool = 1.  Results are identical
- * to the two separate calls. */
-int snnqp_spiking_head_fwd(const snnqp_block_params *p1, const uint8_t *x1,
-                           const int8_t *wq1, const float *scale1,
-                           const float *bias1, uint8_t *spikes1,
-                           const snnqp_block_params *p2, const uint8_t *x2,
-                           const int8_t *wq2, const float *scale2,
-                           const float *bias2, uint8_t *spikes2, void *stream);
-
 /* Plain quantized contraction behind the QuantDense facade (flax_qdense.py:
  * 59-106, lax.dot_general :87-89) and the 1-D k = 4 'SAME' QuantConv facade
  * (flax_qconv.py:131-168 as TCJA uses it, examples/tcja/models.py:52-59,77-84;
@@ -306,7 +289,7 @@ int snnqp_eval_metrics(const float *logits, const int32_t *labels, int B,
                        int classes, float *out2, void *stream);
 
 /* Spike-tile skip statistics of the bit-packed tcgen05 3x3 block: an input
- * box (one strip x one timestep) whose bits are all zero issues no MMAs (its
+ * box (one 16x8 tile x one timestep) whose bits are all zero issues no MMAs (its
  * accumulators are taken as 0; the LIF update still runs).  *skipped / *total =
  * boxes skipped / seen by all launches since the last reset (device-wide
  * counters; the call synchronises with the device). */

@@ -11,7 +11,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # SNNQP_LIB: developer switch for same-box A/B timing of two builds (tools/); the product path is the in-tree .so
 LIB_PATH = os.environ.get("SNNQP_LIB") or os.path.join(_HERE, "libsnnqp.so")
 
-ABI_VERSION = 3          # include/snnqp.h SNNQP_ABI_VERSION (block params carry x_format / y_format / lif_mode)
+ABI_VERSION = 4          # include/snnqp.h SNNQP_ABI_VERSION (block params carry x_format / y_format / lif_mode)
 IMPL_AUTO, IMPL_SIMT, IMPL_TCGEN05 = 0, 1, 2
 SPIKES_U8, SPIKES_BITS = 0, 1
 LIF_EXACT, LIF_FAST, LIF_TENSOR = 0, 1, 2
@@ -68,7 +68,6 @@ SIGNATURES = {
     "snnqp_events_to_frames_packed": (_i, [_vp, _i, _vp, _i64, _i, _i, _i, _i, _i64, _vp, _i, _vp, _vp]),
     "snnqp_slice_nonzeros": (_i, [_vp, _i, _i64, _i64, _vp, _vp]),
     "snnqp_slice_popcount": (_i, [_vp, _i, _i64, _i64, _vp, _vp]),
-    "snnqp_spiking_head_fwd": (_i, [_BP, _vp, _vp, _vp, _vp, _vp, _BP, _vp, _vp, _vp, _vp, _vp, _vp]),
     "snnqp_tile_skip_stats": (_i, [_vp, _vp, _i]),
     "snnqp_qlinear_fwd": (_i, [_vp, _i, _vp, _vp, _i64, _i, _i, _vp, _vp]),
     "snnqp_expand_frames_zsf": (_i, [_vp, _vp, _vp, C.c_uint32, _i64, _i, _vp, _vp]),

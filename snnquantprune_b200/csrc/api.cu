@@ -1,8 +1,8 @@
 // C-ABI entry points of the fused spiking blocks: argument validation and
-// dispatch between the tcgen05 kernels (umma_conv.cu) and the dp4a kernels
-// (simt.cu).  See include/snnqp.h for the contract.
-#include <stdlib.h>
-
+// dispatch between the tcgen05 kernels (umma_conv1.cu / umma_conv1_tc.cu for
+// conv1, umma_conv_t.cu for the 3x3 blocks, umma_att.cu for the attention-
+// weighted blocks and dense layers) and the dp4a kernels (simt.cu).  See
+// include/snnqp.h for the contract.
 #include "common.cuh"
 
 namespace snnqp {
@@ -21,13 +21,7 @@ int launch_vote(const uint8_t *s, int T, int B, int N, int group, int64_t stride
                 int64_t stride_b, float *logits, cudaStream_t st);
 int launch_eval_metrics(const float *logits, const int32_t *labels, int B, int classes,
                         float *out2, cudaStream_t st);
-// umma_conv.cu
-bool umma_conv3x3_supported(const snnqp_block_params &p, const float *att);
-int launch_conv3x3_umma(const snnqp_block_params &p, const uint8_t *x, const int8_t *wq,
-                        const float *scale, const float *bias, uint8_t *spikes, float *u_final,
-                        int32_t *acc_dump, int32_t *counts, cudaStream_t st);
-// umma_conv_t.cu: the pad-free 16 x 8 tile formulation (preferred); umma_conv.cu's strip formulation stays for
-// A/B measurements (SNNQP_CONV_STRIPS=1) and as the conv2 role of the fused head kernel
+// umma_conv_t.cu
 bool umma_conv3x3_tile_supported(const snnqp_block_params &p, const float *att);
 int launch_conv3x3_tile(const snnqp_block_params &p, const uint8_t *x, const int8_t *wq,
                         const float *scale, const float *bias, uint8_t *spikes, float *u_final,
@@ -46,12 +40,6 @@ int launch_dense_umma(const snnqp_block_params &p, const uint8_t *x, const float
 bool umma_conv1_supported(const snnqp_block_params &p, const float *att);
 int launch_conv1_umma(const snnqp_block_params &p, const uint8_t *x, const int8_t *wq4, const float *scale,
                       const float *bias, uint8_t *spikes, float *u_final, int32_t *acc_dump, cudaStream_t st);
-
-// umma_head.cu
-bool umma_head_supported(const snnqp_block_params *p1, const snnqp_block_params *p2);
-int launch_head_fused(const snnqp_block_params *p1, const uint8_t *x1, const int8_t *wq1_quad, const float *scale1,
-                      const float *bias1, uint8_t *y1, const snnqp_block_params *p2, const uint8_t *x2,
-                      const int8_t *wq2, const float *scale2, const float *bias2, uint8_t *y2, cudaStream_t st);
 
 static int check_conv(const snnqp_block_params *p, const void *x, const void *wq,
                       const void *scale, const void *bias, const char *fn) {
@@ -147,47 +135,20 @@ int snnqp_spiking_conv3x3_counts_fwd(const snnqp_block_params *p, const uint8_t 
     if (impl != SNNQP_IMPL_SIMT) return invalid("snnqp_spiking_conv3x3_fwd: impl=%d", p->impl);
     return launch_conv3x3_simt(*p, x, att, wq, scale, bias, spikes, u_final, acc_dump, nullptr, spike_counts, st);
   }
-  static const bool force_strips = getenv("SNNQP_CONV_STRIPS") && atoi(getenv("SNNQP_CONV_STRIPS")) != 0;
-  const bool tile_ok = !force_strips && umma_conv3x3_tile_supported(*p, att);
   if (impl == SNNQP_IMPL_AUTO) {
-    impl = (tile_ok || umma_conv3x3_supported(*p, att)) ? SNNQP_IMPL_TCGEN05 : SNNQP_IMPL_SIMT;
+    impl = umma_conv3x3_tile_supported(*p, att) ? SNNQP_IMPL_TCGEN05 : SNNQP_IMPL_SIMT;
     if (impl == SNNQP_IMPL_SIMT) note_simt_fallback("the 3x3 conv block", p);
   }
-  if (impl == SNNQP_IMPL_TCGEN05 && tile_ok)
-    return launch_conv3x3_tile(*p, x, wq, scale, bias, spikes, u_final, (int32_t *)acc_dump, spike_counts, st);
   if (impl == SNNQP_IMPL_TCGEN05) {
-    if (!umma_conv3x3_supported(*p, att))
-      return unsupported("snnqp_spiking_conv3x3_fwd: tcgen05 path needs Cin=Cout=128, binary/count input, "
-                         "W in {16,32,64}, pool=1 (got Cin=%d Cout=%d W=%d H=%d pool=%d att=%d)",
-                         p->Cin, p->Cout, p->W, p->H, p->pool, att != nullptr);
-    return launch_conv3x3_umma(*p, x, wq, scale, bias, spikes, u_final, (int32_t *)acc_dump, spike_counts, st);
+    if (!umma_conv3x3_tile_supported(*p, att))
+      return unsupported("snnqp_spiking_conv3x3_fwd: tcgen05 path needs Cin=Cout=128, W %% 8 == 0, x strides "
+                         "multiples of 16 bytes (got Cin=%d Cout=%d W=%d x_stride_t=%lld x_stride_b=%lld)",
+                         p->Cin, p->Cout, p->W, (long long)p->x_stride_t, (long long)p->x_stride_b);
+    return launch_conv3x3_tile(*p, x, wq, scale, bias, spikes, u_final, (int32_t *)acc_dump, spike_counts, st);
   }
   if (impl != SNNQP_IMPL_SIMT) return invalid("snnqp_spiking_conv3x3_fwd: impl=%d", p->impl);
   if (any_bits(p)) return bits_need_tcgen05("shape outside the tcgen05 envelope or SNNQP_IMPL_SIMT");
   return launch_conv3x3_simt(*p, x, att, wq, scale, bias, spikes, u_final, acc_dump, nullptr, spike_counts, st);
-}
-
-int snnqp_spiking_head_fwd(const snnqp_block_params *p1, const uint8_t *x1, const int8_t *wq1, const float *scale1,
-                           const float *bias1, uint8_t *spikes1, const snnqp_block_params *p2, const uint8_t *x2,
-                           const int8_t *wq2, const float *scale2, const float *bias2, uint8_t *spikes2, void *stream) {
-  if (int rc = require_device()) return rc;
-  const bool has1 = p1 && p1->B > 0, has2 = p2 && p2->B > 0;
-  if (!has1 && !has2) return invalid("snnqp_spiking_head_fwd: both halves are empty");
-  if (has1) {
-    if (int rc = check_conv(p1, x1, wq1, scale1, bias1, "snnqp_spiking_head_fwd (block 1)")) return rc;
-    if (!spikes1) return invalid("snnqp_spiking_head_fwd: null spikes1");
-  }
-  if (has2) {
-    if (int rc = check_conv(p2, x2, wq2, scale2, bias2, "snnqp_spiking_head_fwd (block 2)")) return rc;
-    if (!spikes2) return invalid("snnqp_spiking_head_fwd: null spikes2");
-  }
-  if (!umma_head_supported(has1 ? p1 : nullptr, has2 ? p2 : nullptr))
-    return unsupported("snnqp_spiking_head_fwd: block 1 must be Cin=2 -> 128 channels, W %% 32 == 0, u8 in / bit-packed "
-                       "out; block 2 128 -> 128 channels at 64x64 with bit-packed input; both standard LIF constants, "
-                       "pool = 1, equal T");
-  // conv1 blob = [Cout][32] tap-major followed by the 4 quad matrices [4][Cout][32]
-  return launch_head_fused(has1 ? p1 : nullptr, x1, has1 ? wq1 + (int64_t)p1->Cout * 32 : nullptr, scale1, bias1, spikes1,
-                           has2 ? p2 : nullptr, x2, wq2, scale2, bias2, spikes2, (cudaStream_t)stream);
 }
 
 int snnqp_qconv3x3_fwd(const snnqp_block_params *p, const uint8_t *x, const int8_t *wq,

@@ -12,7 +12,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 OUT = os.path.join(os.path.dirname(HERE), os.environ.get("SNNQP_BUILD_NAME", "libsnnqp.so"))
-SOURCES = ["runtime.cu", "pack.cu", "simt.cu", "umma_conv.cu", "umma_conv_t.cu", "umma_conv1.cu", "umma_conv1_tc.cu", "umma_head.cu", "umma_att.cu", "diag.cu", "frames.cu", "plain.cu", "api.cu", "xla_ffi_shim.cc"]
+SOURCES = ["runtime.cu", "pack.cu", "simt.cu", "umma_conv_t.cu", "umma_conv1.cu", "umma_conv1_tc.cu", "umma_att.cu", "diag.cu", "frames.cu", "plain.cu", "api.cu", "xla_ffi_shim.cc"]
 HEADERS = ["common.cuh", "ptx.cuh", "tmap.cuh", "epilogue.cuh", os.path.join(ROOT, "include", "snnqp.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

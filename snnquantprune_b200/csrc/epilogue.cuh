@@ -12,6 +12,9 @@ namespace snnqp {
 // bit for bit: (x - u) is rounded once, halving is exact (no subnormals within
 // T steps), and the final add is rounded once in both forms;
 //   (u - 1 >= 0)  ==  (u >= 1)   since an fp32 difference is zero only for equal operands.
+// Both forms must keep two properties of their ordered IEEE compare and NaN-propagating arithmetic: a NaN membrane
+// never spikes and stays NaN.  k_conv3x3_tile's production epilogue relies on it to silence the rows of a partial tile
+// below the image (tests/test_gpu_persistent_schedules.py fires such rows on the bias alone).
 template <bool STD>
 struct LifParams {
   float tau, v_th, v_reset;

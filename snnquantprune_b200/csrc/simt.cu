@@ -3,7 +3,7 @@
 // cross-check kernels (SNNQP_IMPL_SIMT) and the production path for the small
 // layers (conv1's K=18 contraction, conv5/dense1 whose inputs are real-valued,
 // dense2, TCJA); the heavy binary-input convolutions run on tcgen05
-// (umma_conv.cu).  Each kernel keeps the T loop inside, so membrane potentials
+// (umma_conv_t.cu).  Each kernel keeps the T loop inside, so membrane potentials
 // live in registers and never touch HBM between timesteps
 // (reference SpikingBlock scan: spiking_learning.py:441-472).
 #include <stdlib.h>

@@ -23,8 +23,9 @@
 // on that emulation (T = 20, sigmoid-shaped att: ~1e-5 of the conv5
 // neuron-steps undecided, none in dense1).
 //
-//  * k_conv_att_umma : 3x3 conv on 8-wide images (conv5), flat-shift implicit
-//    GEMM exactly as umma_conv.cu, three accumulators per buffer.
+//  * k_conv_att_umma : 3x3 conv on 8-wide images (conv5), implicit GEMM over
+//    strips of full rows read at flat shifts of the (W+2)-pitch box, three
+//    accumulators per buffer.
 //  * k_dense_umma    : [features] x [K] x [(b,t) rows] GEMM with the LIF
 //    recurrence over t running along the accumulator columns of one lane.
 #include <mutex>

@@ -1,19 +1,17 @@
-// Fused SpikingBlock(QuantConv3x3 -> BN -> LIF [-> 2x2 max-pool]) for binary / count inputs, Cin = Cout = 128:
-// the PAD-FREE tiling of the block in umma_conv.cu (same roles, rings, epilogue arithmetic, block-sparse and
-// spike-tile skip paths; reference semantics spiking_learning.py:441-472, flax_qconv.py:158-168,
+// Fused SpikingBlock(QuantConv3x3 -> BN -> LIF [-> 2x2 max-pool]) for binary / count inputs, Cin = Cout = 128, on
+// tcgen05 with a PAD-FREE spatial tiling (reference semantics spiking_learning.py:441-472, flax_qconv.py:158-168,
 // examples/tcja/models.py:101-147).
 //
-// umma_conv.cu walks an image in strips of TH full rows and reads the operand at FLAT shifts of the (W+2)-pitch
-// box, so its MMAs are N = 144 wide of which 128 columns are real outputs (2 pad columns per row, rounded to 16):
-// 11 % of the issued tensor work is pad, its measured 3.9 POP/s is the ceiling of that layout.  Here a work item
-// is a 16 x 8 SPATIAL tile: N = 128 output positions n = g * 8 + j (g = tile row 0..15, j = tile column 0..7).
-// The TMA box is 18 rows x 10 columns x 128 channels (zero-filled halo), 128-byte rows at pitch 10; for tap
-// (kh, kw) tile row g is the 8 consecutive box rows starting at (g + kh) * 10 + kw -- exactly a K-major
+// A work item is a 16 x 8 SPATIAL tile: N = 128 output positions n = g * 8 + j (g = tile row 0..15, j = tile
+// column 0..7).  The TMA box is 18 rows x 10 columns x 128 channels (zero-filled halo), 128-byte rows at pitch 10;
+// for tap (kh, kw) tile row g is the 8 consecutive box rows starting at (g + kh) * 10 + kw -- exactly a K-major
 // 128B-swizzle operand whose 8-row groups are 10 rows (1280 B) apart: the UMMA descriptor's stride-byte-offset
-// carries the image pitch (SBO = 1280 instead of 1024), and because the swizzle is a function of absolute
-// shared-memory address bits (measured in round 1) the groups may start at any 128-byte row.  Every issued MMA
-// column is a real output: 36 MMAs of 128 x 128 x 32 per step instead of 128 x 144 x 32 (-11 % tensor time), the
-// halo re-read drops from 2x to 1.4x, one kernel shape serves every width (W % 8 == 0, H % 16 == 0).
+// carries the box pitch (SBO = 1280 instead of 1024), and because the swizzle is a function of absolute
+// shared-memory address bits (measured in round 1) the groups may start at any 128-byte row.  So every issued MMA
+// column is a real output: 36 MMAs of 128 x 128 x 32 per step.  Reading a strip of full rows at flat shifts of a
+// (W+2)-pitch box instead needs N = 144 for the same 128 outputs (2 pad columns per row, rounded to 16): 11 % more
+// tensor time and a 2x halo re-read against 1.4x here (DESIGN.md section 4.1).  One kernel shape serves every
+// W % 8 == 0 and every even H: the last tile row of an image may be partial (see the epilogue).
 #include <mutex>
 
 #include "common.cuh"
@@ -71,12 +69,11 @@ constexpr int kExpWarps = SNNQP_EXP_WARPS;   // 3 keeps the MMA issuer's SM sub-
 constexpr int kThreadsX = kThreads + kExpWarps * 32;
 constexpr int kPkStages = 6, kPkStageBytes = 2944;   // >= 180 * 16 B, 128-aligned
 constexpr int kTmemCols = 512;
-// Weights (A operand) of the first kTmemTaps taps live in TENSOR MEMORY for the CTA's lifetime: with N = 144 an
-// SS-mode MMA pulls (128 + 144) * 32 B from shared memory per 72 cycles (94 % of the 128 B/cycle port, measured
-// tensor pipe 57 % active); reading A from TMEM leaves 64 B/cycle.  TMEM budget: 2 x 144 accumulator columns +
-// 7 taps x 4 K-steps x 8 columns = 512 exactly.  The last two taps stay in shared memory (32 KB).
-// (template parameters TT = taps in TMEM, ST = input ring depth; production 7 / 4.  Other splits exist to measure
-// how much of the TMEM the layer really needs: tools/time_conv2_variants.py, profiles/r2_conv2_tmem_split.txt)
+// Weights (A operand) of the first SNNQP_T_TAPS taps live in TENSOR MEMORY for the CTA's lifetime, so an MMA reads
+// only its B operand from shared memory: an SS-mode MMA pulls (128 + N) * 32 B per ~64-72 cycles, near the 128 B/cycle
+// port (measured 94 % of it for N = 144 in round 1, tensor pipe 57 % active).  TMEM budget: 2 x 128 accumulator columns
+// + 7 taps x 4 K-steps x 8 columns = 480 of 512.  The other two taps stay in shared memory (32 KB).  How many taps sit
+// in TMEM hardly matters (profiles/r2_conv2_tmem_split.txt).
 constexpr int kAccStride = 128;                 // TMEM column offset of accumulator buffer 1
 constexpr int kACol0 = 2 * kAccStride;          // first TMEM column of the resident weights
 constexpr int smem_bytes_for(int tt, int st, bool xbits = false) {
@@ -390,10 +387,18 @@ k_conv3x3_tile(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
     for (int item = blockIdx.x; item < a.total_items; item += gridDim.x) {
       const int b = item / a.tiles_per_img, tl = item % a.tiles_per_img;
       const int h0 = (tl / a.tiles_x) * kTileH + RT * g, x0 = (tl % a.tiles_x) * kTileW;   // first output row / column of this thread
+      // Partial tile (the last tile row of an image with H % 16 != 0): its rows h0 + r >= H read TMA's zero fill and
+      // run the LIF like the others, but nothing of them may leave the kernel.  H is even and h0 a multiple of 4, so
+      // the two rows of a pooled pair are both inside or both outside.  FAST: such rows start at a NaN membrane, which
+      // never reaches the threshold (epilogue.cuh), so they add nothing to ballots, counts or popcounts; only the
+      // ballot-word store, which is addressed by row, tests the bound.  FAST with u8 output never gets a partial tile
+      // (the host runs those on the generic epilogue), so its stores need no test.  Generic: their spike words are
+      // cleared and their stores skipped.
+      const bool partial = (tl / a.tiles_x) * kTileH + kTileH > a.H;
 #pragma unroll
       for (int r = 0; r < RT; ++r)
 #pragma unroll
-        for (int j = 0; j < 8; ++j) u[r][j] = 0.0f;   // zero carry (spiking_learning.py:464-472)
+        for (int j = 0; j < 8; ++j) u[r][j] = FAST && h0 + r >= a.H ? __int_as_float(0x7fc00000) : 0.0f;   // zero carry (spiking_learning.py:464-472)
       for (int t = 0; t < a.T; ++t, ++step) {
         const uint32_t s = step & 1, ph = (step >> 1) & 1;
         ptx::mbar_wait(acc_full + s, ph);
@@ -441,7 +446,7 @@ k_conv3x3_tile(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
               }
             }
           }
-          if (a.y_bits && lane < 2 * RT) {
+          if (a.y_bits && lane < (partial ? 2 * min(a.H - h0, RT) : 2 * RT)) {
             uint8_t *yw = a.spikes + (int64_t)t * a.y_stride_t + (int64_t)b * a.y_stride_b +
                           ((int64_t)((h0 >> 1) + (lane >> 2)) * Wo + (x0 >> 1) + (lane & 3)) * (kC / 8) + q * 4;
             *reinterpret_cast<uint32_t *>(yw) = mine;
@@ -485,6 +490,7 @@ k_conv3x3_tile(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
             const bool sp = lif.step(u[r][j], __fmaf_rn((float)(int32_t)acc[r][j], sc, bi));
             m[r] |= (sp ? 1u : 0u) << j;
           }
+          if (h0 + r >= a.H) m[r] = 0;
           nspk += __popc(m[r]);
         }
         if (a.counts && nspk) atomicAdd(a.counts + ((int64_t)b * a.T + t) * kC + c, nspk);
@@ -492,6 +498,7 @@ k_conv3x3_tile(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
         if (a.pool) {
 #pragma unroll
           for (int pr = 0; pr < RT / 2; ++pr) {
+            if (h0 + 2 * pr >= a.H) break;
             uint32_t mm = m[2 * pr] | m[2 * pr + 1];
             mm |= mm >> 1;
 #pragma unroll
@@ -500,25 +507,31 @@ k_conv3x3_tile(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
           }
         } else {
 #pragma unroll
-          for (int r = 0; r < RT; ++r)
+          for (int r = 0; r < RT; ++r) {
+            if (h0 + r >= a.H) break;
 #pragma unroll
             for (int j = 0; j < 8; ++j)
               yb[((int64_t)(h0 + r) * Wo + x0 + j) * kC] = (m[r] >> j) & 1u;
+          }
         }
         if (a.acc_dump) {
 #pragma unroll
-          for (int r = 0; r < RT; ++r)
+          for (int r = 0; r < RT; ++r) {
+            if (h0 + r >= a.H) break;
 #pragma unroll
             for (int j = 0; j < 8; ++j)
               a.acc_dump[((((int64_t)t * a.B + b) * a.H + h0 + r) * a.W + x0 + j) * kC + c] = (int32_t)acc[r][j];
+          }
         }
       }
-      if (a.u_final) {
+      if (!FAST && a.u_final) {          // (the host runs FAST only without u_final)
 #pragma unroll
-        for (int r = 0; r < RT; ++r)
+        for (int r = 0; r < RT; ++r) {
+          if (h0 + r >= a.H) break;
 #pragma unroll
           for (int j = 0; j < 8; ++j)
             a.u_final[(((int64_t)b * a.H + h0 + r) * a.W + x0 + j) * kC + c] = u[r][j];
+        }
       }
     }
   }
@@ -538,7 +551,7 @@ k_conv3x3_tile(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
 bool umma_conv3x3_tile_supported(const snnqp_block_params &p, const float *att) {
   if (att) return false;
   if (p.Cin != kC || p.Cout != kC) return false;
-  if (p.W % kTileW != 0 || p.H % kTileH != 0) return false;
+  if (p.W % kTileW != 0) return false;       // any (even) H: the last tile row may be partial
   if (p.x_stride_t % 16 || p.x_stride_b % 16) return false;
   return true;
 }
@@ -597,7 +610,7 @@ int launch_conv3x3_tile(const snnqp_block_params &p, const uint8_t *x, const int
   UmmaArgs a;
   a.T = p.T; a.B = p.B; a.H = p.H; a.W = p.W;
   a.tiles_x = p.W / kTileW;
-  a.tiles_per_img = a.tiles_x * (p.H / kTileH);
+  a.tiles_per_img = a.tiles_x * ((p.H + kTileH - 1) / kTileH);
   a.total_items = p.B * a.tiles_per_img;
   a.y_stride_t = p.y_stride_t; a.y_stride_b = p.y_stride_b;
   a.tau = p.tau; a.v_th = p.v_threshold; a.v_reset = p.v_reset;
@@ -619,7 +632,9 @@ int launch_conv3x3_tile(const snnqp_block_params &p, const uint8_t *x, const int
   a.spikes = spikes; a.u_final = u_final; a.acc_dump = acc_dump; a.counts = counts; a.wq = wq;
 
   const int grid = a.total_items < sm_count() ? a.total_items : sm_count();
-  const bool fast = p.tau == 2.0f && p.v_threshold == 1.0f && p.v_reset == 0.0f && p.pool && !u_final && !acc_dump;
+  // FAST with u8 output stores unconditionally: a partial last tile row takes the generic epilogue there (same bits)
+  const bool fast = p.tau == 2.0f && p.v_threshold == 1.0f && p.v_reset == 0.0f && p.pool && !u_final && !acc_dump &&
+                    (a.y_bits || p.H % kTileH == 0);
   if (a.y_bits && !fast)
     return unsupported("tcgen05 conv: bit-packed output needs the production variant (standard LIF constants, pool = 1, "
                        "no u_final / acc_dump)");
@@ -651,13 +666,16 @@ int launch_conv3x3_tile(const snnqp_block_params &p, const uint8_t *x, const int
 
 }  // namespace snnqp
 
-namespace snnqp {
-int tile_kernel_skip_stats(unsigned long long *h, bool reset) {
-  SNNQP_CUDA(cudaMemcpyFromSymbol(h, g_tile_skip_t, 2 * sizeof(unsigned long long)));
+extern "C" int snnqp_tile_skip_stats(int64_t *skipped, int64_t *total, int reset) {
+  using namespace snnqp;
+  if (int rc = require_device()) return rc;
+  unsigned long long h[2] = {0, 0};
+  SNNQP_CUDA(cudaMemcpyFromSymbol(h, g_tile_skip_t, sizeof(h)));
+  if (skipped) *skipped = (int64_t)h[0];
+  if (total) *total = (int64_t)h[1];
   if (reset) {
     const unsigned long long z[2] = {0, 0};
     SNNQP_CUDA(cudaMemcpyToSymbol(g_tile_skip_t, z, sizeof(z)));
   }
   return SNNQP_OK;
 }
-}  // namespace snnqp

@@ -28,50 +28,11 @@ from ._lib import BlockParams
 from .pack import PackedCextNet
 
 
-class _HeadPipe:
-  """Chunk pipeline of the head (conv1 -> conv2 -> conv3).  Un-fused: the three launches per chunk.  Fused
-  (``engine.fused_head``): conv1 of the pushed chunk shares one persistent kernel with conv2 of the previous chunk
-  (two s1 buffers in flight); ``finish`` drains the last chunk."""
-
-  def __init__(self, eng, ws, collect=None):
-    self.eng, self.ws, self.collect = eng, ws, collect
-    self.fused = eng.fused_head and collect is None
-    self.prev = None
-    self.i = 0
-
-  def _s1(self, i):
-    return self.ws["s1"] if (i & 1) == 0 else self.ws["s1b"]
-
-  def push(self, frames_chunk, b0, n):
-    eng, ws = self.eng, self.ws
-    if not self.fused:
-      eng._head(frames_chunk, b0, n, ws, self.collect)
-      return
-    H, C = eng.pk.H, eng.pk.channels
-    pb0, pn = self.prev if self.prev else (0, 0)
-    eng._head_fused(frames_chunk, n, self._s1(self.i), self._s1(self.i - 1), pn, ws["s2"])
-    if pn:
-      eng._conv(2, ws["s2"][:pn], ws["s3"][pb0:pb0 + pn], pn, H // 4, C, 1)
-    self.prev = (b0, n)
-    self.i += 1
-
-  def finish(self):
-    if not self.fused or not self.prev:
-      return
-    eng, ws = self.eng, self.ws
-    H, C = eng.pk.H, eng.pk.channels
-    pb0, pn = self.prev
-    eng._head_fused(None, 0, None, self._s1(self.i - 1), pn, ws["s2"])
-    eng._conv(2, ws["s2"][:pn], ws["s3"][pb0:pb0 + pn], pn, H // 4, C, 1)
-    self.prev = None
-
-
 class CextNetEngine:
   def __init__(self, packed: PackedCextNet, impl: int = _lib.IMPL_AUTO,
                tau: float = 2.0, v_threshold: float = 1.0, v_reset: float = 0.0,
                chunk: int = 296, device="cuda", lif_mode: int = _lib.LIF_TENSOR,
-               packed_spikes: Optional[bool] = None, fused_head: Optional[bool] = None,
-               track_densities: bool = False):
+               packed_spikes: Optional[bool] = None, track_densities: bool = False):
     """``packed_spikes``: conv1 -> conv2 -> conv3 -> conv4 exchange bit-packed spikes (SNNQP_SPIKES_BITS, 8x fewer
     bytes; tcgen05 kernels only, the default unless impl == IMPL_SIMT).  ``lif_mode`` concerns conv1, the block bound by its LIF epilogue
     (every other block always runs the reference's op order): LIF_EXACT = the reference's op order, bit-identical to
@@ -91,11 +52,6 @@ class CextNetEngine:
     if packed_spikes and not in_envelope:
       raise ValueError("packed_spikes needs the tcgen05 kernels: H = 128, 128 channels, impl != IMPL_SIMT")
     self.packed_spikes = in_envelope if packed_spikes is None else bool(packed_spikes)
-    # conv1 of chunk k+1 and conv2 of chunk k in one persistent kernel (snnqp_spiking_head_fwd); needs the bit-packed
-    # layout and the standard LIF constants.  Off by default: see DESIGN.md section 4.6 for the measured state.
-    self.fused_head = False if fused_head is None else bool(fused_head)
-    if self.fused_head and not self.packed_spikes:
-      raise ValueError("fused_head needs packed_spikes")
     self.tau, self.v_th, self.v_reset = tau, v_threshold, v_reset
     self.chunk = chunk
     self.device = torch.device(device)
@@ -121,7 +77,6 @@ class CextNetEngine:
     Cs = C // 8 if self.packed_spikes else C                     # bytes per position of s1 / s2 / s3
     ws = {
         "s1": torch.empty((Bc, T, H // 2, H // 2, Cs), **u8),    # per chunk
-        "s1b": torch.empty((Bc, T, H // 2, H // 2, Cs), **u8) if self.fused_head else None,   # second chunk in flight
         "s2": torch.empty((Bc, T, H // 4, H // 4, Cs), **u8),    # per chunk
         "s3": torch.empty((B, T, H // 8, H // 8, Cs), **u8),     # whole batch from here on
         "p4": torch.empty((B, T, H // 16, H // 16, C), **u8),
@@ -213,11 +168,9 @@ class CextNetEngine:
     # head: conv1 -> conv2 -> conv3, chunk by chunk
     if self.track_densities:
       ws["dens"].zero_()
-    pipe = _HeadPipe(self, ws, collect)
     for b0 in range(0, B, Bc):
       n = min(Bc, B - b0)
-      pipe.push(frames[b0:b0 + n], b0, n)
-    pipe.finish()
+      self._head(frames[b0:b0 + n], b0, n, ws, collect)
     self._tail(B, ws, logits, collect)
 
   def _head(self, frames_chunk, b0, n, ws, collect=None):
@@ -246,23 +199,6 @@ class CextNetEngine:
     """SNNQP_SPIKES_BITS (..., C/8) uint8 -> SNNQP_SPIKES_U8 (..., C) uint8 (bit c & 7 of byte c >> 3)."""
     sh = torch.arange(8, device=x.device, dtype=torch.uint8)
     return ((x.unsqueeze(-1) >> sh) & 1).reshape(tuple(x.shape[:-1]) + (x.shape[-1] * 8,))
-
-  def _head_fused(self, frames_chunk, n1, s1_out, s1_in, n2, s2_out):
-    """One launch of snnqp_spiking_head_fwd: conv1 on ``frames_chunk`` (n1 samples, may be 0) and conv2 on ``s1_in``
-    (n2 samples, may be 0)."""
-    L, P = _lib.lib(), _lib.ptr
-    pk, H, C = self.pk, self.pk.H, self.pk.channels
-    p1 = p2 = None
-    x1 = y1 = x2 = y2 = None
-    if n1:
-      x1, y1 = frames_chunk, s1_out[:n1]
-      p1 = self._bp(n1, H, 2, C, x1, y1, 1)
-    if n2:
-      x2, y2 = s1_in[:n2], s2_out[:n2]
-      p2 = self._bp(n2, H // 2, C, C, x2, y2, 1)
-    l1, l2 = pk.convs[0], pk.convs[1]
-    _lib.check(L.snnqp_spiking_head_fwd(p1, P(x1), P(l1.wq), P(l1.scale), P(l1.bias), P(y1),
-                                        p2, P(x2), P(l2.wq), P(l2.scale), P(l2.bias), P(y2), _lib.stream()))
 
   def _tail(self, B, ws, logits, collect=None):
     pk = self.pk
@@ -381,7 +317,6 @@ class CextNetEngine:
     logits = torch.empty((B, pk.num_classes), device=self.device, dtype=torch.float32)
     self._copy_stream.wait_stream(cur)
     done = []
-    pipe = _HeadPipe(self, ws)
     for i, (b0, n) in enumerate(self.host_chunks(B)):
       buf = ws["stage"][i & 1][:n]
       if i >= 2:
@@ -391,11 +326,10 @@ class CextNetEngine:
         ready = torch.cuda.Event()
         ready.record(self._copy_stream)
       cur.wait_event(ready)
-      pipe.push(buf, b0, n)
+      self._head(buf, b0, n, ws)
       ev = torch.cuda.Event()
       ev.record(cur)
       done.append(ev)
-    pipe.finish()
     self._tail(B, ws, logits)
     if out_host is not None:
       out_host.copy_(logits, non_blocking=True)
@@ -434,7 +368,6 @@ class CextNetEngine:
     logits = torch.empty((B, pk.num_classes), device=self.device, dtype=torch.float32)
     self._copy_stream.wait_stream(cur)
     done = []
-    pipe = _HeadPipe(self, ws)
     for i, (b0, n) in enumerate(chunks):
       bm, bo, vals, vbase, nblk = zb.chunk(b0, b0 + n)
       dbm, dbo, dv = ws["zsf"][i & 1]
@@ -449,11 +382,10 @@ class CextNetEngine:
         ready.record(self._copy_stream)
       cur.wait_event(ready)
       zsf_expand(dbm, dbo, dv, vbase, nblk, zb.value_bits, buf)
-      pipe.push(buf, b0, n)
+      self._head(buf, b0, n, ws)
       ev = torch.cuda.Event()
       ev.record(cur)
       done.append(ev)
-    pipe.finish()
     self._tail(B, ws, logits)
     if out_host is not None:
       out_host.copy_(logits, non_blocking=True)
@@ -497,7 +429,6 @@ class CextNetEngine:
     logits = torch.empty((B, pk.num_classes), device=self.device, dtype=torch.float32)
     self._copy_stream.wait_stream(cur)
     done = []
-    pipe = _HeadPipe(self, ws)
     for i, (b0, n) in enumerate(chunks):
       words, offs, base = eb.chunk(b0, b0 + n)
       dev, doff = ev[i & 1]
@@ -513,11 +444,10 @@ class CextNetEngine:
       events_to_frames_packed(dev, doff[:n + 1], eb.format, pk.T, eb.sensor_wh, resolution_scale, out=buf,
                               max_events_per_sample=eb.max_events_per_sample, event_base=base,
                               n_saturated=n_saturated)
-      pipe.push(buf, b0, n)
+      self._head(buf, b0, n, ws)
       e = torch.cuda.Event()
       e.record(cur)
       done.append(e)
-    pipe.finish()
     self._tail(B, ws, logits)
     if out_host is not None:
       out_host.copy_(logits, non_blocking=True)

@@ -281,7 +281,7 @@ def test_spiking_conv1_counts_bit_exact(cuda_lib, oracle_lib, shape, bits, pool)
 @pytest.mark.parametrize("shape,bits,pool,prune", [
     ((3, 2, 16, 16, 128), 8, True, 0.5), ((2, 1, 32, 32, 128), 4, True, 0.8),
     ((2, 2, 64, 64, 128), 8, True, 0.5), ((3, 1, 16, 16, 128), 2, False, 0.9),
-    ((1, 1, 8, 8, 128), 8, False, 0.0)])
+    ((1, 1, 8, 8, 128), 8, False, 0.0), ((2, 3, 22, 24, 128), 8, False, 0.5)])
 def test_spiking_conv_binary_bit_exact(cuda_lib, oracle_lib, impl, shape, bits, pool, prune):
   T, B, H, W, Cin = shape
   p0 = BlockParams(); p0.T, p0.B, p0.H, p0.W, p0.Cin, p0.Cout, p0.pool, p0.impl = T, B, H, W, Cin, 128, int(pool), impl
@@ -839,42 +839,7 @@ def test_spike_tile_skip_on_structured_frames(cuda_lib):
     got = CextNetEngine(pk, lif_mode=_lib.LIF_EXACT, packed_spikes=True).forward(frd).cpu().numpy()
     _lib.check(cuda_lib.snnqp_tile_skip_stats(ctypes.byref(sk), ctypes.byref(tot), 1))
     assert np.array_equal(got, want), name
-    assert tot.value == B * T * (32 + 8 + 2)               # strips of conv2 / conv3 / conv4 per sample-step
+    assert tot.value == B * T * (32 + 8 + 2)               # 16x8 tiles of conv2 / conv3 / conv4 per sample-step
     rates[name] = sk.value / tot.value
   assert rates["blob"] >= 0.5 and rates["iid"] == 0.0, rates
 
-
-@pytest.mark.parametrize("lif_mode", [_lib.LIF_EXACT, _lib.LIF_FAST])
-def test_fused_head_equals_separate_launches(cuda_lib, lif_mode):
-  """snnqp_spiking_head_fwd (conv1 of chunk k+1 and conv2 of chunk k in one persistent kernel, TMEM / shared memory /
-  registers carved between the two roles) gives exactly the spikes of the two separate launches: per-launch check
-  of both halves, conv1-only and conv2-only launches, then whole forwards over several (ragged) chunk schedules."""
-  from snnquantprune_b200 import CextNetEngine, pack_cextnet
-  bits, T, H, B = 8, 20, 128, 40
-  v = synthetic.make_variables(bits=bits, prune_percentage=0.5, T=T, H=H, seed=1)
-  pk = pack_cextnet(v, bits, T, H, device=DEV)
-  fr = dev(synthetic.make_frames(B, T, H, H, seed=8))
-  sep = CextNetEngine(pk, chunk=B, lif_mode=lif_mode, fused_head=False)
-  fus = CextNetEngine(pk, chunk=B, lif_mode=lif_mode, fused_head=True)
-  C = pk.channels
-  # separate launches
-  s1 = torch.empty((B, T, H // 2, H // 2, C // 8), device=DEV, dtype=torch.uint8)
-  s2 = torch.empty((B, T, H // 4, H // 4, C // 8), device=DEV, dtype=torch.uint8)
-  sep._conv(0, fr, s1, B, H, 2, 1)
-  sep._conv(1, s1, s2, B, H // 2, C, 1)
-  # fused: both halves at once on different sample ranges (conv1 on all B, conv2 on the first 17 samples of s1)
-  f1 = torch.zeros_like(s1); f2 = torch.zeros_like(s2)
-  fus._head_fused(fr, B, f1, s1, 17, f2)
-  assert torch.equal(f1, s1), "conv1 half"
-  assert torch.equal(f2[:17], s2[:17]), "conv2 half"
-  # each half alone
-  f1.zero_(); f2.zero_()
-  fus._head_fused(fr[:5], 5, f1, None, 0, None)
-  assert torch.equal(f1[:5], s1[:5])
-  fus._head_fused(None, 0, None, s1, B, f2)
-  assert torch.equal(f2, s2)
-  # whole forward, several chunk schedules (single chunk, equal chunks, ragged tail)
-  want = sep.forward(fr)
-  for chunk in (B, 20, 37, 16):
-    got = CextNetEngine(pk, chunk=chunk, lif_mode=lif_mode, fused_head=True).forward(fr)
-    assert torch.equal(got, want), chunk

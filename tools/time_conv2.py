@@ -20,5 +20,5 @@ torch.cuda.synchronize(); e0.record()
 for _ in range(n_it): fn()
 e1.record(); torch.cuda.synchronize()
 us = e0.elapsed_time(e1) / n_it * 1e3
-print(f"conv2 B={B} strips={os.environ.get('SNNQP_CONV_STRIPS', '0')} packed={int(eng.packed_spikes)}: {us:9.1f} us = {us / B:6.3f} us/sample = "
+print(f"conv2 B={B} packed={int(eng.packed_spikes)}: {us:9.1f} us = {us / B:6.3f} us/sample = "
       f"{24.16e9 * B / us / 1e6:7.1f} TOP/s, checksum {int(s2.sum().item())}")

@@ -28,10 +28,5 @@ timeit(f"tcja ({B})", lambda: eng._tcja(0, B, H // 8, None, ws["cnt4"], ws["att4
 timeit(f"conv5 att ({B})", lambda: eng._conv(4, ws["p4"], ws["p5"], B, H // 16, C, 1, att=ws["att4"], counts=ws["cnt5"]))
 timeit(f"dense1 att ({B})", lambda: eng._dense(eng.pk.dense1, B, ws["p5"].view(B, T, -1), ws["att5"], ws["d1"]))
 timeit(f"dense2 ({B})", lambda: eng._dense(eng.pk.dense2, B, ws["d1"], None, ws["d2"]))
-if eng.fused_head:
-  s1b = ws["s1b"][:n]
-  timeit(f"head kernel: conv1 only ({n})", lambda: eng._head_fused(fr[:n], n, s1b, None, 0, None))
-  timeit(f"head kernel: conv2 only ({n})", lambda: eng._head_fused(None, 0, None, s1, n, s2))
-  timeit(f"head kernel: conv1 || conv2 ({n})", lambda: eng._head_fused(fr[:n], n, s1b, s1, n, s2))
 timeit(f"forward ({B})", lambda: eng.forward(fr), 3)
 timeit(f"forward_graph ({B})", lambda: eng.forward_graph(fr), 3)
