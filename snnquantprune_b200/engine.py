@@ -34,7 +34,10 @@ class CextNetEngine:
                chunk: int = 296, device="cuda", lif_mode: int = _lib.LIF_TENSOR,
                packed_spikes: Optional[bool] = None, track_densities: bool = False):
     """``packed_spikes``: conv1 -> conv2 -> conv3 -> conv4 exchange bit-packed spikes (SNNQP_SPIKES_BITS, 8x fewer
-    bytes; tcgen05 kernels only, the default unless impl == IMPL_SIMT).  ``lif_mode`` concerns conv1, the block bound by its LIF epilogue
+    bytes).  Only the production epilogues of the tcgen05 kernels emit them, and those hard-code the standard LIF
+    constants (tau = 2, v_threshold = 1, v_reset = 0): the default is on at H = 128, 128 channels, impl != IMPL_SIMT
+    and standard constants, off otherwise; True with other constants raises ValueError (the generic epilogues that
+    run such constants emit SNNQP_SPIKES_U8).  ``lif_mode`` concerns conv1, the block bound by its LIF epilogue
     (every other block always runs the reference's op order): LIF_EXACT = the reference's op order, bit-identical to
     the oracle; LIF_FAST = single-rounding fma on the CUDA cores (membranes within 1 ulp per step, 12 flipped spikes in
     3.1e9); LIF_TENSOR (default) = the leak runs on the tensor core (tcgen05.mma scale-input-d, membranes resident in
@@ -51,7 +54,11 @@ class CextNetEngine:
     in_envelope = impl != _lib.IMPL_SIMT and packed.H == 128 and packed.channels == 128
     if packed_spikes and not in_envelope:
       raise ValueError("packed_spikes needs the tcgen05 kernels: H = 128, 128 channels, impl != IMPL_SIMT")
-    self.packed_spikes = in_envelope if packed_spikes is None else bool(packed_spikes)
+    std_lif = (tau, v_threshold, v_reset) == (2.0, 1.0, 0.0)
+    if packed_spikes and not std_lif:
+      raise ValueError(f"packed_spikes needs the standard LIF constants (tau = 2, v_threshold = 1, v_reset = 0); got "
+                       f"tau = {tau}, v_threshold = {v_threshold}, v_reset = {v_reset}")
+    self.packed_spikes = (in_envelope and std_lif) if packed_spikes is None else bool(packed_spikes)
     self.tau, self.v_th, self.v_reset = tau, v_threshold, v_reset
     self.chunk = chunk
     self.device = torch.device(device)

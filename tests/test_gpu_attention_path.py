@@ -258,7 +258,7 @@ def test_band_on_emulated_attention_path(oracle_lib):
 
 
 # ================================================================================= GPU: conv5 and dense1 ====
-def launch_conv(lib, x, att_d, packed, impl, *, pool, tau=2.0, batch_major=True, dumps=True):
+def launch_conv(lib, x, att_d, packed, impl, *, pool, tau=2.0, batch_major=True, dumps=True, v_th=1.0, v_reset=0.0):
   """snnqp_spiking_conv3x3_counts_fwd on x (T, B, H, 8, 128) u8 (device copy batch-major or time-major) with att_d a
   device view (T, B, 128) of any strides.  Returns spikes (T, B, Ho, Wo, C), and with dumps u_T, acc, counts."""
   T, B, H, W, C = x.shape
@@ -279,7 +279,7 @@ def launch_conv(lib, x, att_d, packed, impl, *, pool, tau=2.0, batch_major=True,
   p.y_stride_t, p.y_stride_b = spikes.stride(0), spikes.stride(1)
   p.att_stride_t, p.att_stride_b = att_d.stride(0), att_d.stride(1)
   p.att_mod = C
-  p.tau, p.v_threshold, p.v_reset = tau, 1.0, 0.0
+  p.tau, p.v_threshold, p.v_reset = tau, v_th, v_reset
   p.pool, p.impl = int(pool), impl
   _lib.check(lib.snnqp_spiking_conv3x3_counts_fwd(p, P(xs), P(att_d), P(packed.wq), P(packed.scale), P(packed.bias),
                                                   P(spikes), P(u), P(acc), P(cnt), _lib.stream()))
@@ -309,15 +309,17 @@ def first_diff(name, got, want):
   return f"{name}: {len(d)} elements differ, first {d[:4].tolist()}"
 
 
-def check_conv(lib, x, att, q, packed, scale, bias, impl, *, tau=2.0, layout="bt", pad=0, batch_major=True):
+def check_conv(lib, x, att, q, packed, scale, bias, impl, *, tau=2.0, layout="bt", pad=0, batch_major=True, v_th=1.0,
+               v_reset=0.0):
   """Un-pooled launch with every dump against the emulation, then the pooled production variant (no dumps)."""
   emu = ar.conv_att_tc_acc(x, att, q) if impl == _lib.IMPL_TCGEN05 else ar.conv_att_simt_acc(x, att, q)
-  s_e, u_e = ref_int.lif_from_acc(emu, scale, bias, tau)
+  s_e, u_e = ref_int.lif_from_acc(emu, scale, bias, tau, v_th, v_reset)
   att_d = att_device(att, layout, pad)
-  s, u, acc, cnt = launch_conv(lib, x, att_d, packed, impl, pool=False, tau=tau, batch_major=batch_major)
+  lif = dict(tau=tau, v_th=v_th, v_reset=v_reset)
+  s, u, acc, cnt = launch_conv(lib, x, att_d, packed, impl, pool=False, batch_major=batch_major, **lif)
   msgs = [first_diff("acc", acc, emu), first_diff("spikes", s, s_e), first_diff("u_final", u, u_e),
           first_diff("spike_counts", cnt, s_e.sum(axis=(2, 3), dtype=np.int32).transpose(1, 0, 2))]
-  (sp,) = launch_conv(lib, x, att_d, packed, impl, pool=True, tau=tau, batch_major=batch_major, dumps=False)
+  (sp,) = launch_conv(lib, x, att_d, packed, impl, pool=True, batch_major=batch_major, dumps=False, **lif)
   msgs.append(first_diff("pooled production spikes", sp, ref_int.maxpool2_u8(s_e)))
   msgs = [m for m in msgs if m]
   assert not msgs, msgs
@@ -363,7 +365,7 @@ def test_conv_att_simt_bit_exact(cuda_lib, oracle_lib, T, B, H, layout, pad, tau
   check_conv(cuda_lib, x, edge_att(rng, T, B), q, packed, scale, bias, _lib.IMPL_SIMT, tau=tau, layout=layout, pad=pad)
 
 
-def launch_dense(lib, x, att_d, packed, N, impl, dumps=True):
+def launch_dense(lib, x, att_d, packed, N, impl, dumps=True, tau=2.0, v_th=1.0, v_reset=0.0):
   """snnqp_spiking_dense_fwd, x (T, B, K) u8 batch-major on the device, att_d a (T, B, 128) device view."""
   T, B, K = x.shape
   xs = dev(np.swapaxes(x, 0, 1))
@@ -376,7 +378,7 @@ def launch_dense(lib, x, att_d, packed, N, impl, dumps=True):
   p.y_stride_t, p.y_stride_b = spikes.stride(0), spikes.stride(1)
   p.att_stride_t, p.att_stride_b = att_d.stride(0), att_d.stride(1)
   p.att_mod = 128
-  p.tau, p.v_threshold, p.v_reset = 2.0, 1.0, 0.0
+  p.tau, p.v_threshold, p.v_reset = tau, v_th, v_reset
   p.impl = impl
   _lib.check(lib.snnqp_spiking_dense_fwd(p, P(xs), P(att_d), P(packed.wq), P(packed.scale), P(packed.bias), P(spikes),
                                          P(u), P(acc), _lib.stream()))
@@ -384,15 +386,17 @@ def launch_dense(lib, x, att_d, packed, N, impl, dumps=True):
   return [spikes.cpu().numpy()] + ([u.cpu().numpy(), acc.cpu().numpy()] if dumps else [])
 
 
-def check_dense(lib, x, att, q, packed, scale, bias, impl, emu_impl=None, pad=0, layout="bt"):
+def check_dense(lib, x, att, q, packed, scale, bias, impl, emu_impl=None, pad=0, layout="bt", tau=2.0, v_th=1.0,
+                v_reset=0.0):
   emu_impl = impl if emu_impl is None else emu_impl
   K, N = q.shape
   att_k = np.tile(att, (1, 1, K // 128))
   emu = ar.dense_att_tc_acc(x, att_k, q) if emu_impl == _lib.IMPL_TCGEN05 else ar.dense_att_simt_acc(x, att_k, q)
-  s_e, u_e = ref_int.lif_from_acc(emu, scale, bias)
+  s_e, u_e = ref_int.lif_from_acc(emu, scale, bias, tau, v_th, v_reset)
   att_d = att_device(att, layout, pad)
-  s, u, acc = launch_dense(lib, x, att_d, packed, N, impl)
-  (sp,) = launch_dense(lib, x, att_d, packed, N, impl, dumps=False)
+  lif = dict(tau=tau, v_th=v_th, v_reset=v_reset)
+  s, u, acc = launch_dense(lib, x, att_d, packed, N, impl, **lif)
+  (sp,) = launch_dense(lib, x, att_d, packed, N, impl, dumps=False, **lif)
   msgs = [first_diff("acc", acc, emu), first_diff("spikes", s, s_e), first_diff("u_final", u, u_e),
           first_diff("production spikes", sp, s_e)]
   msgs = [m for m in msgs if m]

@@ -126,7 +126,7 @@ def test_fold_affine_bit_exact(cuda_lib):
 
 # ------------------------------------------------------- fused conv block ----
 def run_conv(lib, x_tb, wq, scale, bias, Cout, pool, impl, att=None, tau=2.0, batch_major=False, counts=None,
-             dumps=True, x_bits=False, y_bits=False, lif_mode=0, popcount=None):
+             dumps=True, x_bits=False, y_bits=False, lif_mode=0, popcount=None, v_th=1.0, v_reset=0.0):
   """x_tb: numpy (T,B,H,W,Cin) u8.  Calls snnqp_spiking_conv3x3_fwd through the
   C-ABI; returns numpy (spikes (T,B,Ho,Wo,C), u (B,H,W,C), acc (T,B,H,W,C)).
   ``popcount``: optional int32 CUDA tensor [B][T] passed as y_popcount."""
@@ -152,7 +152,7 @@ def run_conv(lib, x_tb, wq, scale, bias, Cout, pool, impl, att=None, tau=2.0, ba
     attd = dev(att)
     p.att_stride_t, p.att_stride_b = attd.stride(0), attd.stride(1)
   p.att_mod = Cin
-  p.tau, p.v_threshold, p.v_reset = tau, 1.0, 0.0
+  p.tau, p.v_threshold, p.v_reset = tau, v_th, v_reset
   p.pool, p.impl = int(pool), impl
   p.x_format, p.y_format, p.lif_mode = int(x_bits), int(y_bits), lif_mode
   if popcount is not None:
@@ -437,7 +437,7 @@ def test_qconv_plain_forward(cuda_lib, oracle_lib):
 
 
 # ------------------------------------------------------------ dense / tcja ----
-def run_dense(lib, x, wq, scale, bias, N, att=None, att_mod=0, impl=_lib.IMPL_SIMT):
+def run_dense(lib, x, wq, scale, bias, N, att=None, att_mod=0, impl=_lib.IMPL_SIMT, tau=2.0, v_th=1.0, v_reset=0.0):
   """x: numpy (T,B,K); the device copy is batch-major [B][T][K] (rows (b,t) contiguous)."""
   T, B, K = x.shape
   xs = dev(np.ascontiguousarray(np.swapaxes(x, 0, 1)))
@@ -452,7 +452,7 @@ def run_dense(lib, x, wq, scale, bias, N, att=None, att_mod=0, impl=_lib.IMPL_SI
   if att is not None:
     attd = dev(att); p.att_stride_t, p.att_stride_b = attd.stride(0), attd.stride(1)
   p.att_mod = att_mod
-  p.tau, p.v_threshold, p.v_reset = 2.0, 1.0, 0.0
+  p.tau, p.v_threshold, p.v_reset = tau, v_th, v_reset
   p.impl = impl
   _lib.check(lib.snnqp_spiking_dense_fwd(p, P(xs), P(attd), P(wq), P(scale), P(bias), P(spikes), P(u), P(acc),
                                          _lib.stream()))
@@ -622,8 +622,17 @@ def test_network_layerwise_teacher_forced_and_float_path(cuda_lib, oracle_lib):
   assert np.array_equal(tb("d2"), co["d2"])
   assert np.array_equal(logits, lo)
   # reference-order float path, free running
+  check_free_running_vs_float_path(c, logits, v, fr, bits)
+
+
+def check_free_running_vs_float_path(c, logits, v, fr, bits, tau=2.0, v_th=1.0, v_reset=0.0):
+  """The instrumented engine forward (collect dict c, logits) against the reference-order float path run free with
+  the same LIF constants: per block <= 1e-4 flipped spikes, every conv membrane within 1e-5 unless a counted flip sits
+  upstream, logits within one output-spike quantum per counted flip (up to 16)."""
+  T = fr.shape[1]
+  tb = lambda k: np.ascontiguousarray(np.swapaxes(c[k].cpu().numpy(), 0, 1))
   cf = {}
-  lf = ref_snn.cextnet_forward(v, fr, bits, collect=cf)
+  lf = ref_snn.cextnet_forward(v, fr, bits, tau, v_th, v_reset, collect=cf)
   nflip = 0
   for k, kf in (("s1", "pool1"), ("s2", "pool2"), ("s3", "pool3"), ("s4", "conv4_spikes"),
                 ("s5", "conv5_spikes"), ("d1", "dense1_spikes"), ("d2", "dense2_spikes")):

@@ -227,6 +227,36 @@ def test_host_chunk_schedule_covers_batch_and_respects_cap():
       assert body == sorted(body)
 
 
+LIF_CONSTANTS_OFF_DEFAULT = [(1.7, 0.8, 0.1), (3.0, 1.0, 0.0), (2.0, 0.75, 0.0), (2.0, 1.0, 0.125), (2.0, 0.5, -0.25),
+                             (2.0, -0.5, 0.0), (4.0, 0.75, 0.25), (0.5, 1.0, 1.2)]
+
+
+def test_engine_packed_spikes_needs_standard_lif_constants():
+  """Bit-packed spikes come only from the production epilogues, which hard-code tau = 2, v_threshold = 1, v_reset = 0;
+  the conv launchers refuse bit-packed output with any other constants.  So at the reference geometry the engine's
+  default must turn packing off for such constants (else every production forward fails at conv1), and an explicit
+  packed_spikes=True with them is refused in the constructor.  Only packed.H and packed.channels are read there."""
+  from types import SimpleNamespace
+  from snnquantprune_b200 import _lib
+  from snnquantprune_b200.engine import CextNetEngine
+  ref_geom = SimpleNamespace(H=128, channels=128)
+  assert CextNetEngine(ref_geom, device="cpu").packed_spikes
+  assert CextNetEngine(ref_geom, tau=2.0, v_threshold=1.0, v_reset=0.0, device="cpu").packed_spikes
+  assert not CextNetEngine(ref_geom, impl=_lib.IMPL_SIMT, device="cpu").packed_spikes
+  assert not CextNetEngine(SimpleNamespace(H=64, channels=128), device="cpu").packed_spikes
+  for tau, vth, vr in LIF_CONSTANTS_OFF_DEFAULT:
+    eng = CextNetEngine(ref_geom, tau=tau, v_threshold=vth, v_reset=vr, device="cpu")
+    assert eng.packed_spikes is False, (tau, vth, vr)
+    assert (eng.tau, eng.v_th, eng.v_reset) == (tau, vth, vr)
+    assert CextNetEngine(ref_geom, tau=tau, v_threshold=vth, v_reset=vr, device="cpu",
+                         packed_spikes=False).packed_spikes is False
+    with pytest.raises(ValueError, match="standard LIF constants"):
+      CextNetEngine(ref_geom, tau=tau, v_threshold=vth, v_reset=vr, device="cpu", packed_spikes=True)
+  # the envelope check still comes first: outside it, packing is refused whatever the constants
+  with pytest.raises(ValueError, match="tcgen05"):
+    CextNetEngine(SimpleNamespace(H=64, channels=128), device="cpu", packed_spikes=True)
+
+
 def test_cextnet_engine_cache_key_follows_content():
   """The facade caches its packed engine on a content digest: an in-place edit of the variable tree (what
   import_torch_tcja / re-calibration do) must change the key, an untouched tree must not."""
